@@ -13,9 +13,11 @@ A "step" = one pass of the hot path over one batch of synthetic frames per GPU:
             peer-memory stores per step by default, the NCCL all_gather with TSMDET_GATHER=nccl.
 Prints ONE JSON line (rank 0).  `value` = frames/s with inputs resident in HBM; `e2e` = the same through the
 host-buffer API (one pinned collated input buffer H2D + one packed result buffer D2H per step, inside the timed
-region).  Both are the MEDIAN of `--repeats` timed regions of exactly K steps each.  After the timed regions the last
-step's results are verified against the oracle (`verified`), the unmodified reference CUDA extension is timed on
-the same inputs (`ref_cuda_baseline`) and the other BASELINE configs are measured (`secondary`).
+region).  Each is measured over exactly K = `--steps` timed steps (split into `--repeats` regions, one by default).
+After the timed regions the last step's results are verified against the oracle (`verified`), the unmodified reference
+CUDA extension is timed on the same inputs (`ref_cuda_baseline`) and the other BASELINE configs are measured
+(`secondary`).  `--dump-outputs DIR` writes the arrays the last timed device-resident step returned as DIR/<name>.npy; the
+inputs and weights are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -284,7 +286,7 @@ def main():
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=50)
     ap.add_argument("--warmup", type=int, default=8)
-    ap.add_argument("--repeats", type=int, default=5, help="timed regions of K steps each; the median is reported")
+    ap.add_argument("--repeats", type=int, default=1, help="timed regions the K steps are split into")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--precision", default=os.environ.get("TSMDET_BENCH_PRECISION", "bf16"), choices=["fp32", "bf16", "tf32"])
     ap.add_argument("--depth", type=int, default=int(os.environ.get("TSMDET_BENCH_DEPTH", "8")),
@@ -292,6 +294,8 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip verify / ref_cuda_baseline / secondary configs")
     ap.add_argument("--profile-kernels", action="store_true", help="per-kernel CUDA-event breakdown to stderr")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the results of the last timed step as DIR/<name>.npy (float32, integers as float64)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
@@ -351,20 +355,25 @@ def main():
     host_ms = []
 
     def timed_repeats(submit):
-        """`--repeats` regions of exactly K steps, each bracketed by barrier + synchronize; per region the MAX over
-        ranks; returns (sorted list of region ms, median)."""
+        """Exactly K steps in `--repeats` regions, each bracketed by barrier + synchronize; per region the MAX over
+        ranks; returns (list of region ms, total ms)."""
+        regions = max(1, min(args.repeats, args.steps))
         out = []
-        for _ in range(max(1, args.repeats)):
+        for i in range(regions):
             barrier()
-            t = torch.tensor([timed(submit, args.steps)], dtype=torch.float64, device=dev)
+            steps = args.steps // regions + (i < args.steps % regions)
+            t = torch.tensor([timed(submit, steps)], dtype=torch.float64, device=dev)
             barrier()
             if world > 1:
                 dist.all_reduce(t, op=dist.ReduceOp.MAX)
             out.append(float(t))
-        out.sort()
-        return out, out[len(out) // 2]
+        return out, sum(out)
 
-    dev_step = lambda: runner.submit_device(lane_inputs, gather=gather, pre=flush)  # noqa: E731
+    last = {}
+
+    def dev_step():
+        last["res"] = runner.submit_device(lane_inputs, gather=gather, pre=flush)[1]
+
     host_step = lambda: runner.submit_host(gather=gather, pre=flush)  # noqa: E731
 
     for _ in range(depth):  # prime every lane once (graph upload, first collective) whatever --warmup is
@@ -398,8 +407,13 @@ def main():
     t_wall = time.perf_counter()
     dev_regions, ms_total = timed_repeats(dev_step)
     wall = time.perf_counter() - t_wall
-    launches = (_lib.launch_count - l0) // max(1, args.repeats)
+    launches = _lib.launch_count - l0
     clocks = sampler.stop()
+    # copied before any later step can replay the last timed step's graph and overwrite its results
+    # (`packed` / `det_packed` are left out: they are the same bytes as features | xyz | det | det_num)
+    dumped = ({k: v.cpu().numpy().astype(np.float32 if v.is_floating_point() else np.float64)
+               for k, v in last["res"].items() if k not in ("packed", "det_packed")}
+              if args.dump_outputs and rank == 0 else None)
     for _ in range(depth + args.warmup):
         host_step()
     runner.sync()
@@ -464,7 +478,7 @@ def main():
                 "host_affinity": affinity},
         "gpu_launches": int(launches), "clocks": clocks, "roofline": roof,
         "fps_ms_per_cloud": next((k["ms"] for k in kernels if k["name"] == "fps_L1"), None),
-        "repeats": {"n": len(dev_regions), "statistic": "median", "ms_per_region_device": dev_regions,
+        "repeats": {"n": len(dev_regions), "statistic": "sum", "ms_per_region_device": dev_regions,
                     "ms_per_region_e2e": e2e_regions},
         "execution": {"mlp_precision": args.precision, "pipeline_depth": depth,
                       "graph": "one CUDA graph per step (FPS chain, query+MLP, NMS on 3 concurrent streams); "
@@ -519,6 +533,10 @@ def main():
                                           f"kernels + torch-CPU fp32 MLP + oracle rotated NMS"}
     elif rank == 0:
         line["cpu_baseline"] = None
+    if dumped is not None:  # 8.8 MB for the 16-frame step
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dumped.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     if rank == 0:
         print(json.dumps(line), flush=True)
     if world > 1:
