@@ -230,6 +230,21 @@ int tsmdet_stack_group_points_grad(int b, int m, int c, int n, int nsample, cons
  *      n_total = N.  The reference's block size is 1024 for every cloud, and so is the tie rule here. */
 int tsmdet_stack_farthest_point_sampling(int n_total, int batch_size, const float* xyz, float* temp,
                                          const int* xyz_batch_cnt, int* idxs, const int* num_sampled_points, void* stream);
+/* ref: pointnet2_api.cpp:15 ball_query_wrapper (ball_query.cpp:25-45; ball_query_gpu.cu:15-62): new_xyz (M,3) and
+ *      xyz (N,3) stacked, new_xyz_batch_cnt / xyz_batch_cnt (B) i32 on the device, n_total = N.  idx (M,nsample) i32
+ *      ZEROED by the caller receives the first min(hits, nsample) frame-local indices with d2 < radius * radius in
+ *      ascending order, the remaining slots repeating the first hit; a centre without hits gets only idx[p,0] = -1.
+ *      idx_cnt (M) i32, optional (NULL), receives min(hits, nsample).  global_rows = 1: frame start + index instead,
+ *      and all-zero rows for centres without hits (the fused stacked SA scale's input).  No host synchronisation;
+ *      TSMDET_BQ_ALGO=brute skips the per-frame grids. */
+int tsmdet_stack_ball_query(int b, int m, int n_total, float radius, int nsample, const float* new_xyz,
+                            const int* new_xyz_batch_cnt, const float* xyz, const int* xyz_batch_cnt, int* idx,
+                            int* idx_cnt, int global_rows, void* stream);
+/* Stacked features (N,C) f32 -> the fused SA kernels' feature rows (N,Cp), zero padded: precision 1 = bf16
+ * (Cp = round_up(C,8), round to nearest even), 2 = tf32 as f32 bit patterns (Cp = round_up(C,4), round half away) --
+ * the rounding the kernels apply to (B,C,N) planes themselves.  Pass the result as features_t of
+ * tsmdet_sa_mlp_maxpool_packed_p with B = 1. */
+int tsmdet_stack_feature_rows(int precision, int n, int c, const float* features, void* rows, void* stream);
 
 /* ---------------------------------------------------------------- IoU / NMS ---------
  * boxes (N,7) f32 [x,y,z,dx,dy,dz,heading] on the device.

@@ -19,6 +19,11 @@
 // A cloud whose points pile up in one cell (> kMaxCell per cell: degenerate input, or r comparable to the
 // whole cloud) is flagged and left to the brute-force kernels of ball_query.cu, which skip flagged-OK
 // clouds -- no host synchronisation either way.
+//
+// Stacked (ragged) frames, pointnet2_stack's ball query: bq_grid_build_ragged_kernel builds one grid per frame over its
+// own points and bq_grid_query16_ragged_kernel / bq_grid_merge_ragged_kernel run the same search cores
+// (grid_query16_core, grid_merge_core); they differ only in finding the centre's frame and in the write-back (first-hit
+// padding, -1 for an empty ball).  Unusable frames go to stack_ball_query_brute_kernel (stack_ball_query.cu).
 #include <math.h>
 #include <string.h>
 
@@ -27,9 +32,10 @@
 
 namespace tsm {
 
-__global__ void __launch_bounds__(1024, 1)
-    bq_grid_build_kernel(int n, float rout, const float* __restrict__ xyz_all, int* __restrict__ hdr_all,
-                         int* __restrict__ cell_start_all, float4* sorted_tmp_all, float4* __restrict__ sorted_all) {
+// The grid of ONE cloud of n points, built by a whole 1024-thread CTA (the batch and the ragged build kernels below
+// differ only in where a cloud's points and outputs start).
+__device__ __forceinline__ void grid_build_cloud(int n, float rout, const float* __restrict__ xyz, int* const hdr,
+                                                 int* const cell_start, float4* const tmp, float4* const sorted) {
     extern __shared__ __align__(16) unsigned char dyn[];
     uint32_t* const hist = reinterpret_cast<uint32_t*>(dyn);  // [kGridCells]
     __shared__ float red[6][32];
@@ -37,12 +43,6 @@ __global__ void __launch_bounds__(1024, 1)
     __shared__ uint32_t wmaxc[32];
     constexpr int T = 1024, NW = 32;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const int cloud = blockIdx.x;
-    const float* __restrict__ xyz = xyz_all + (size_t)cloud * n * 3;
-    int* const hdr = hdr_all + (size_t)cloud * kHdrInts;
-    int* const cell_start = cell_start_all + (size_t)cloud * (kGridCells + 1);
-    float4* const tmp = sorted_tmp_all + (size_t)cloud * n;
-    float4* const sorted = sorted_all + (size_t)cloud * n;
 
     // (1) bounding box
     const float inf = __int_as_float(0x7f800000);
@@ -193,23 +193,34 @@ __global__ void __launch_bounds__(1024, 1)
     }
 }
 
-template <bool DILATED>
-__global__ void __launch_bounds__(256)
-    bq_grid_merge_kernel(int b, int n, int m, float rin2, float rout2, int nsample, const float* __restrict__ new_xyz,
-                         const int* __restrict__ hdr_all, const int* __restrict__ cell_start_all,
-                         const float4* __restrict__ sorted_all, int* __restrict__ idx_cnt, int* __restrict__ idx) {
-    const int lane = threadIdx.x & 31;
-    const long long wid = (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-    if (wid >= (long long)b * m) return;
-    const int cloud = (int)(wid / m);
-    const GridHdr h = *reinterpret_cast<const GridHdr*>(hdr_all + (size_t)cloud * kHdrInts);
-    if (!h.ok) return;
-    const int* __restrict__ cell_start = cell_start_all + (size_t)cloud * (kGridCells + 1);
-    const float4* __restrict__ sorted = sorted_all + (size_t)cloud * n;
-    const float* q = new_xyz + (size_t)wid * 3;
-    const float cx = __ldg(q), cy = __ldg(q + 1), cz = __ldg(q + 2);
-    int* const row = idx + (size_t)wid * nsample;
+__global__ void __launch_bounds__(1024, 1)
+    bq_grid_build_kernel(int n, float rout, const float* __restrict__ xyz_all, int* __restrict__ hdr_all,
+                         int* __restrict__ cell_start_all, float4* sorted_tmp_all, float4* __restrict__ sorted_all) {
+    const int cloud = blockIdx.x;
+    grid_build_cloud(n, rout, xyz_all + (size_t)cloud * n * 3, hdr_all + (size_t)cloud * kHdrInts,
+                     cell_start_all + (size_t)cloud * (kGridCells + 1), sorted_tmp_all + (size_t)cloud * n,
+                     sorted_all + (size_t)cloud * n);
+}
 
+// Stacked clouds: frame f holds points start[f] .. start[f+1]-1 of xyz (N,3); its sorted records carry frame-local
+// indices.
+__global__ void __launch_bounds__(1024, 1)
+    bq_grid_build_ragged_kernel(float rout, const int* __restrict__ start, const float* __restrict__ xyz,
+                                int* __restrict__ hdr_all, int* __restrict__ cell_start_all, float4* sorted_tmp,
+                                float4* __restrict__ sorted) {
+    const int f = blockIdx.x;
+    const int s = start[f];
+    grid_build_cloud(start[f + 1] - s, rout, xyz + (size_t)s * 3, hdr_all + (size_t)f * kHdrInts,
+                     cell_start_all + (size_t)f * (kGridCells + 1), sorted_tmp + s, sorted + s);
+}
+
+// The `nsample` smallest hit indices (ascending) of the centre (cx, cy, cz) in one cloud's grid, written to row[0..cnt)
+// as index + off by the lanes that own them; returns cnt.  Lane l < 27 walks the sorted list of one neighbour cell up
+// to its next hit; the warp repeatedly takes the smallest pending index (redux.sync.min).
+template <bool DILATED>
+__device__ __forceinline__ int grid_merge_core(int lane, const GridHdr& h, const int* __restrict__ cell_start,
+                                               const float4* __restrict__ sorted, float cx, float cy, float cz, float rin2,
+                                               float rout2, int nsample, int* const row, int off) {
     // lane l < 27 owns neighbour cell (dz, dy, dx) = (l / 9 - 1, l / 3 % 3 - 1, l % 3 - 1)
     int head = 0, end = 0;
     if (lane < 27) {
@@ -243,11 +254,32 @@ __global__ void __launch_bounds__(256)
         const uint32_t mn = __reduce_min_sync(FULL, cur);
         if (mn == 0xffffffffu) break;
         if (cur == mn) {
-            row[cnt] = (int)mn;
+            row[cnt] = (int)mn + off;
             advance();
         }
         ++cnt;
     }
+    return cnt;
+}
+
+template <bool DILATED>
+__global__ void __launch_bounds__(256)
+    bq_grid_merge_kernel(int b, int n, int m, float rin2, float rout2, int nsample, const float* __restrict__ new_xyz,
+                         const int* __restrict__ hdr_all, const int* __restrict__ cell_start_all,
+                         const float4* __restrict__ sorted_all, int* __restrict__ idx_cnt, int* __restrict__ idx) {
+    const int lane = threadIdx.x & 31;
+    const long long wid = (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (wid >= (long long)b * m) return;
+    const int cloud = (int)(wid / m);
+    const GridHdr h = *reinterpret_cast<const GridHdr*>(hdr_all + (size_t)cloud * kHdrInts);
+    if (!h.ok) return;
+    const int* __restrict__ cell_start = cell_start_all + (size_t)cloud * (kGridCells + 1);
+    const float4* __restrict__ sorted = sorted_all + (size_t)cloud * n;
+    const float* q = new_xyz + (size_t)wid * 3;
+    const float cx = __ldg(q), cy = __ldg(q + 1), cz = __ldg(q + 2);
+    int* const row = idx + (size_t)wid * nsample;
+
+    const int cnt = grid_merge_core<DILATED>(lane, h, cell_start, sorted, cx, cy, cz, rin2, rout2, nsample, row, 0);
     // counts + cyclic padding (row[p] = row[p mod cnt]); rows without hits are zeroed
     __syncwarp();
     if (lane == 0) idx_cnt[wid] = cnt;
@@ -349,34 +381,15 @@ __global__ void __launch_bounds__(256)
     }
 }
 
-// nsample <= 16 * R (R = 1, 2): the same algorithm with HALF a warp per centre (two centres per warp).  At the first SA layer a ball
-// holds one or two points (the centre itself and maybe a neighbour) and a few dozen candidates, so a whole warp per centre
-// is mostly fixed cost: ncu counts 346 warp-instructions per centre at 80 % issue utilisation -- the kernel is
-// instruction-bound.  A lane owns neighbour cells gl and gl + 16 (candidates may be numbered in any order: the result is
-// the nsample smallest hit indices whatever the order), collectives run on the half-warp's own member mask, lane e of the
-// half ends up with the e-th (and, R = 2, the (e + 16)-th) smallest hit, and the grid is (centres, clouds) so that no
-// 64-bit division is needed.
+// The half-warp search of bq_grid_query16_kernel for the centre (cx, cy, cz) in one cloud's grid: lane e of the half
+// ends with the (e + 16 i)-th smallest hit index in best[i] (NONE past the last); returns the number of hits kept
+// (<= nsample).
 template <bool DILATED, int R>
-__global__ void __launch_bounds__(256)
-    bq_grid_query16_kernel(int n, int m, float rin2, float rout2, int nsample, const float* __restrict__ new_xyz,
-                           const int* __restrict__ hdr_all, const int* __restrict__ cell_start_all,
-                           const float4* __restrict__ sorted_all, int* __restrict__ idx_cnt, int* __restrict__ idx) {
+__device__ __forceinline__ int grid_query16_core(int gl, unsigned gmask, const GridHdr& h, const int* __restrict__ cell_start,
+                                                 const float4* __restrict__ sorted, float cx, float cy, float cz, float rin2,
+                                                 float rout2, int nsample, uint32_t (&best)[R]) {
     constexpr int K = 4;
     constexpr uint32_t NONE = 0xffffffffu;
-    const int lane = threadIdx.x & 31, gl = lane & 15;
-    const unsigned gmask = 0xffffu << (lane & 16);
-    const int cloud = blockIdx.y;
-    const int centre = (blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5)) * 2 + (lane >> 4);
-    if (centre >= m) return;  // (a whole half-warp leaves together)
-    const GridHdr h = *reinterpret_cast<const GridHdr*>(hdr_all + (size_t)cloud * kHdrInts);
-    if (!h.ok) return;
-    const int* __restrict__ cell_start = cell_start_all + (size_t)cloud * (kGridCells + 1);
-    const float4* __restrict__ sorted = sorted_all + (size_t)cloud * n;
-    const size_t wid = (size_t)cloud * m + centre;
-    const float* q = new_xyz + wid * 3;
-    const float cx = __ldg(q), cy = __ldg(q + 1), cz = __ldg(q + 2);
-    int* const row = idx + wid * nsample;
-
     const int qx = grid_q(cx, h.lo[0], h.inv[0], h.n[0]), qy = grid_q(cy, h.lo[1], h.inv[1], h.n[1]),
               qz = grid_q(cz, h.lo[2], h.inv[2], h.n[2]);
     int beg[2] = {0, 0}, len[2] = {0, 0};
@@ -400,7 +413,7 @@ __global__ void __launch_bounds__(256)
     const int total = __shfl_sync(gmask, incl, 15, 16);
     const int excl_len0 = ((incl - loc) << 16) | len[0];  // (both < 2^15: a cell holds <= kMaxCell points, 27 cells)
 
-    uint32_t best[R];  // lane e of the half: the (e + 16 i)-th smallest hit so far
+    // lane e of the half: the (e + 16 i)-th smallest hit so far
 #pragma unroll
     for (int i = 0; i < R; ++i) best[i] = NONE;
     for (int base = 0; base < total; base += 16 * K) {
@@ -452,6 +465,37 @@ __global__ void __launch_bounds__(256)
     int cnt = 0;
 #pragma unroll
     for (int i = 0; i < R; ++i) cnt += __popc(__ballot_sync(gmask, best[i] != NONE) & gmask);
+    return cnt;
+}
+
+// nsample <= 16 * R (R = 1, 2): the same algorithm with HALF a warp per centre (two centres per warp).  At the first SA layer a ball
+// holds one or two points (the centre itself and maybe a neighbour) and a few dozen candidates, so a whole warp per centre
+// is mostly fixed cost: ncu counts 346 warp-instructions per centre at 80 % issue utilisation -- the kernel is
+// instruction-bound.  A lane owns neighbour cells gl and gl + 16 (candidates may be numbered in any order: the result is
+// the nsample smallest hit indices whatever the order), collectives run on the half-warp's own member mask, lane e of the
+// half ends up with the e-th (and, R = 2, the (e + 16)-th) smallest hit, and the grid is (centres, clouds) so that no
+// 64-bit division is needed.
+template <bool DILATED, int R>
+__global__ void __launch_bounds__(256)
+    bq_grid_query16_kernel(int n, int m, float rin2, float rout2, int nsample, const float* __restrict__ new_xyz,
+                           const int* __restrict__ hdr_all, const int* __restrict__ cell_start_all,
+                           const float4* __restrict__ sorted_all, int* __restrict__ idx_cnt, int* __restrict__ idx) {
+    const int lane = threadIdx.x & 31, gl = lane & 15;
+    const unsigned gmask = 0xffffu << (lane & 16);
+    const int cloud = blockIdx.y;
+    const int centre = (blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5)) * 2 + (lane >> 4);
+    if (centre >= m) return;  // (a whole half-warp leaves together)
+    const GridHdr h = *reinterpret_cast<const GridHdr*>(hdr_all + (size_t)cloud * kHdrInts);
+    if (!h.ok) return;
+    const int* __restrict__ cell_start = cell_start_all + (size_t)cloud * (kGridCells + 1);
+    const float4* __restrict__ sorted = sorted_all + (size_t)cloud * n;
+    const size_t wid = (size_t)cloud * m + centre;
+    const float* q = new_xyz + wid * 3;
+    const float cx = __ldg(q), cy = __ldg(q + 1), cz = __ldg(q + 2);
+    int* const row = idx + wid * nsample;
+
+    uint32_t best[R];
+    const int cnt = grid_query16_core<DILATED, R>(gl, gmask, h, cell_start, sorted, cx, cy, cz, rin2, rout2, nsample, best);
     if (gl == 0) idx_cnt[wid] = cnt;
     // row[p] = hit[p mod cnt] (cyclic padding); rows without hits are zeroed
 #pragma unroll
@@ -464,6 +508,86 @@ __global__ void __launch_bounds__(256)
             if (src >= 16) val = hi;
         }
         if (p < nsample) row[p] = cnt ? (int)val : 0;
+    }
+}
+
+// ---- stacked (ragged) clouds, pointnet2_stack's ball_query_kernel_stack contract: centre p belongs to frame
+// stack_frame_of(p); its row holds the first min(hits, nsample) frame-local hit indices in ascending order, the
+// remaining slots repeat the FIRST hit, and a row without hits gets only row[0] = -1 (the caller zeroed the rest).
+// global_rows != 0 (the fused SA path): frame start + index instead, and all-zero rows without hits.  idx_cnt may be
+// null.  Frames whose grid is unusable are left to stack_ball_query_brute_kernel (stack_ball_query.cu).
+template <int R>
+__global__ void __launch_bounds__(256)
+    bq_grid_query16_ragged_kernel(int b, int m, float rout2, int nsample, const float* __restrict__ new_xyz,
+                                  const int* __restrict__ mstart, const int* __restrict__ nstart,
+                                  const int* __restrict__ hdr_all, const int* __restrict__ cell_start_all,
+                                  const float4* __restrict__ sorted_all, int* __restrict__ idx_cnt, int* __restrict__ idx,
+                                  int global_rows) {
+    const int lane = threadIdx.x & 31, gl = lane & 15;
+    const unsigned gmask = 0xffffu << (lane & 16);
+    const int centre = (blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5)) * 2 + (lane >> 4);
+    if (centre >= m) return;  // (a whole half-warp leaves together)
+    const int f = stack_frame_of(centre, b, mstart);
+    const GridHdr h = *reinterpret_cast<const GridHdr*>(hdr_all + (size_t)f * kHdrInts);
+    if (!h.ok) return;
+    const int start = __ldg(nstart + f);
+    const float* q = new_xyz + (size_t)centre * 3;
+    const float cx = __ldg(q), cy = __ldg(q + 1), cz = __ldg(q + 2);
+    int* const row = idx + (size_t)centre * nsample;
+
+    uint32_t best[R];
+    const int cnt = grid_query16_core<false, R>(gl, gmask, h, cell_start_all + (size_t)f * (kGridCells + 1),
+                                                sorted_all + start, cx, cy, cz, 0.f, rout2, nsample, best);
+    if (idx_cnt && gl == 0) idx_cnt[centre] = cnt;
+    const int off = global_rows ? start : 0;
+#pragma unroll
+    for (int i = 0; i < R; ++i) {
+        const int p = gl + 16 * i;
+        const int src = p < cnt ? p : 0;  // past the hits: the first hit
+        uint32_t val = __shfl_sync(gmask, best[0], src & 15, 16);
+        if (R > 1) {
+            const uint32_t hi = __shfl_sync(gmask, best[R - 1], src & 15, 16);
+            if (src >= 16) val = hi;
+        }
+        if (p < nsample) {
+            if (cnt) row[p] = (int)val + off;
+            else if (global_rows) row[p] = 0;
+            else if (p == 0) row[0] = -1;
+        }
+    }
+}
+
+// nsample > 32: one warp per centre (the merge walk of bq_grid_merge_kernel), same contract as above.
+__global__ void __launch_bounds__(256)
+    bq_grid_merge_ragged_kernel(int b, int m, float rout2, int nsample, const float* __restrict__ new_xyz,
+                                const int* __restrict__ mstart, const int* __restrict__ nstart,
+                                const int* __restrict__ hdr_all, const int* __restrict__ cell_start_all,
+                                const float4* __restrict__ sorted_all, int* __restrict__ idx_cnt, int* __restrict__ idx,
+                                int global_rows) {
+    const int lane = threadIdx.x & 31;
+    const int centre = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (centre >= m) return;
+    const int f = stack_frame_of(centre, b, mstart);
+    const GridHdr h = *reinterpret_cast<const GridHdr*>(hdr_all + (size_t)f * kHdrInts);
+    if (!h.ok) return;
+    const int start = __ldg(nstart + f);
+    const float* q = new_xyz + (size_t)centre * 3;
+    const float cx = __ldg(q), cy = __ldg(q + 1), cz = __ldg(q + 2);
+    int* const row = idx + (size_t)centre * nsample;
+    const int off = global_rows ? start : 0;
+
+    const int cnt = grid_merge_core<false>(lane, h, cell_start_all + (size_t)f * (kGridCells + 1), sorted_all + start,
+                                           cx, cy, cz, 0.f, rout2, nsample, row, off);
+    __syncwarp();  // row[0] (the first hit) was written by whichever lane owned it
+    if (idx_cnt && lane == 0) idx_cnt[centre] = cnt;
+    if (cnt == 0) {
+        if (global_rows)
+            for (int p = lane; p < nsample; p += 32) row[p] = 0;
+        else if (lane == 0)
+            row[0] = -1;
+    } else {
+        const int first = row[0];
+        for (int p = cnt + lane; p < nsample; p += 32) row[p] = first;
     }
 }
 
@@ -533,6 +657,49 @@ int tsm_ball_query_grid(bool dilated, int b, int n, int m, float rin, float rout
         else
             bq_grid_merge_kernel<false><<<blocks, 256, 0, stream>>>(b, n, m, rin2, rout2, nsample, new_xyz, hdr,
                                                                     cell_start, sorted, idx_cnt, idx);
+    }
+    TSM_LAUNCH_CHECK();
+    *grid_hdr = hdr;
+    return TSM_OK;
+}
+
+int tsm_stack_ball_query_grid(int b, int m, int n_total, float radius, int nsample, const float* new_xyz,
+                              const int* mstart, const int* nstart, const float* xyz, int* idx, int* idx_cnt,
+                              int global_rows, cudaStream_t stream, const int** grid_hdr) {
+    using namespace tsm;
+    *grid_hdr = nullptr;
+    // radius * radius is what the query compares: a negative radius is its absolute value, 0 / NaN hit nothing (every
+    // frame then goes to the brute-force kernel)
+    const float rout = fabsf(radius);
+    if (!(rout > 0.f) || n_total <= 0) return TSM_OK;
+    const size_t hdr_bytes = ((size_t)b * kHdrInts * sizeof(int) + 255) & ~(size_t)255;
+    const size_t cs_bytes = ((size_t)b * (kGridCells + 1) * sizeof(int) + 255) & ~(size_t)255;
+    const size_t pts_bytes = ((size_t)n_total * sizeof(float4) + 255) & ~(size_t)255;
+    void* base = nullptr;
+    int rc = tsm_scratch_get(9, hdr_bytes + cs_bytes + 2 * pts_bytes, stream, &base);
+    if (rc != TSM_OK) return rc;
+    unsigned char* p = static_cast<unsigned char*>(base);
+    int* hdr = reinterpret_cast<int*>(p);
+    int* cell_start = reinterpret_cast<int*>(p + hdr_bytes);
+    float4* tmp = reinterpret_cast<float4*>(p + hdr_bytes + cs_bytes);
+    float4* sorted = reinterpret_cast<float4*>(p + hdr_bytes + cs_bytes + pts_bytes);
+    const size_t dyn = (size_t)kGridCells * sizeof(uint32_t);
+    TSM_CUDA_TRY(cudaFuncSetAttribute(bq_grid_build_ragged_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
+    bq_grid_build_ragged_kernel<<<b, 1024, dyn, stream>>>(rout, nstart, xyz, hdr, cell_start, tmp, sorted);
+    TSM_LAUNCH_CHECK();
+    const float rout2 = radius * radius;  // f32 product, as ball_query_gpu.cu (stack):25
+    if (nsample <= 32) {
+        const unsigned blocks = (unsigned)((m + 15) / 16);
+        if (nsample <= 16)
+            bq_grid_query16_ragged_kernel<1><<<blocks, 256, 0, stream>>>(b, m, rout2, nsample, new_xyz, mstart, nstart, hdr,
+                                                                         cell_start, sorted, idx_cnt, idx, global_rows);
+        else
+            bq_grid_query16_ragged_kernel<2><<<blocks, 256, 0, stream>>>(b, m, rout2, nsample, new_xyz, mstart, nstart, hdr,
+                                                                         cell_start, sorted, idx_cnt, idx, global_rows);
+    } else {
+        bq_grid_merge_ragged_kernel<<<(unsigned)((m + 7) / 8), 256, 0, stream>>>(b, m, rout2, nsample, new_xyz, mstart, nstart,
+                                                                                 hdr, cell_start, sorted, idx_cnt, idx,
+                                                                                 global_rows);
     }
     TSM_LAUNCH_CHECK();
     *grid_hdr = hdr;

@@ -20,9 +20,27 @@ __device__ __forceinline__ int grid_q(float v, float lo, float inv, int n) {
     return min(max(__float2int_rd(__fmul_rn(__fsub_rn(v, lo), inv)), 0), n - 1);
 }
 
+// Frame of row p of a stacked (ragged) batch, as ball_query_kernel_stack finds it: the first k with
+// p < M0 + ... + Mk, the search stopping at b - 1.  mstart = the (b + 1) exclusive prefix sums of the counts.
+__device__ __forceinline__ int stack_frame_of(int p, int b, const int* __restrict__ mstart) {
+    int lo = 0, hi = b - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if (p < __ldg(mstart + mid + 1)) hi = mid; else lo = mid + 1;
+    }
+    return lo;
+}
+
 }  // namespace tsm
 
 // Builds the grid of every cloud on `stream` (scratch tag `tag`): cells at least 1.01 * rout wide, or -- rout < 0 --
 // sized for about two points per cell.  Returns device pointers into the scratch buffer.
 int tsm_grid_build(int b, int n, float rout, const float* xyz, cudaStream_t stream, int tag, const int** hdr,
                    const int** cell_start, const float4** sorted);
+
+// Stacked clouds: one grid per frame over its own points (nstart / mstart = the (b + 1) exclusive prefix sums of the
+// point / centre counts, on the device); answers every centre of a frame whose grid is usable.  *grid_hdr receives the
+// per-frame headers (word 9 = usable; nullptr: no grid was built) for the brute-force kernel.
+int tsm_stack_ball_query_grid(int b, int m, int n_total, float radius, int nsample, const float* new_xyz,
+                              const int* mstart, const int* nstart, const float* xyz, int* idx, int* idx_cnt,
+                              int global_rows, cudaStream_t stream, const int** grid_hdr);

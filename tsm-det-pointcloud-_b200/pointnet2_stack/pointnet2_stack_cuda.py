@@ -15,6 +15,15 @@ def _chk(*tensors):
             raise ValueError("must be a contiguous tensor")
 
 
+def ball_query_wrapper(B, M, radius, nsample, new_xyz, new_xyz_batch_cnt, xyz, xyz_batch_cnt, idx):
+    """ref ball_query.cpp:25-45: new_xyz (M,3), xyz (N,3) stacked, counts (B) int32, idx (M,nsample) int32 zeroed by
+    the caller -> frame-local rows, first hit repeated past the hits, idx[p,0] = -1 for a centre without hits"""
+    _chk(new_xyz, new_xyz_batch_cnt, xyz, xyz_batch_cnt, idx)
+    call("tsmdet_stack_ball_query", B, M, xyz.shape[0], float(radius), nsample, ptr(new_xyz), ptr(new_xyz_batch_cnt),
+         ptr(xyz), ptr(xyz_batch_cnt), ptr(idx), None, 0, stream_ptr(xyz.device))
+    return 1
+
+
 def voxel_query_wrapper(M, R1, R2, R3, nsample, radius, z_range, y_range, x_range, new_xyz, xyz, new_coords,
                         point_indices, idx, cnt_unique):
     """ref voxel_query.cpp:27-46"""

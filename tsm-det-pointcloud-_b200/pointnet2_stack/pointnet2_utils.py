@@ -1,13 +1,45 @@
-"""``GroupingOperation`` / ``StackFarthestPointSampling`` / ``FarthestPointSampling`` of
-``/root/reference/pcdet/ops/pointnet2/pointnet2_stack/pointnet2_utils.py`` (:48-105, 158-222) on the sm_100a kernels:
-same signatures, argument checks and returns (the ball-query, 3-NN and vector-pool ops of that file are not on the
-path of the shipped model and are not part of this package)."""
+"""``BallQuery`` / ``QueryAndGroup`` / ``GroupingOperation`` / ``StackFarthestPointSampling`` /
+``FarthestPointSampling`` of ``/root/reference/pcdet/ops/pointnet2/pointnet2_stack/pointnet2_utils.py`` (:10-105,
+158-222) on the sm_100a kernels: same signatures, argument checks and returns (the 3-NN and vector-pool ops of that
+file are not part of this package)."""
 from __future__ import annotations
 
 import torch
+import torch.nn as nn
 from torch.autograd import Function
 
 from . import pointnet2_stack_cuda as pointnet2
+
+
+class BallQuery(Function):
+    """ref :10-45"""
+
+    @staticmethod
+    def forward(ctx, radius: float, nsample: int, xyz: torch.Tensor, xyz_batch_cnt: torch.Tensor,
+                new_xyz: torch.Tensor, new_xyz_batch_cnt):
+        """xyz (N1+N2..., 3), xyz_batch_cnt (B), new_xyz (M1+M2..., 3), new_xyz_batch_cnt (B)
+        -> (idx (M1+M2..., nsample) int32 frame-local rows, empty_ball_mask (M1+M2...) bool); rows of empty balls are 0"""
+        assert new_xyz.is_contiguous()
+        assert new_xyz_batch_cnt.is_contiguous()
+        assert xyz.is_contiguous()
+        assert xyz_batch_cnt.is_contiguous()
+
+        B = xyz_batch_cnt.shape[0]
+        M = new_xyz.shape[0]
+        idx = torch.zeros((M, nsample), dtype=torch.int32, device=new_xyz.device)
+        pointnet2.ball_query_wrapper(B, M, radius, nsample, new_xyz, new_xyz_batch_cnt, xyz, xyz_batch_cnt, idx)
+        empty_ball_mask = idx[:, 0] == -1
+        idx[empty_ball_mask] = 0
+        ctx.mark_non_differentiable(idx)
+        ctx.mark_non_differentiable(empty_ball_mask)
+        return idx, empty_ball_mask
+
+    @staticmethod
+    def backward(ctx, a=None, b=None):
+        return None, None, None, None, None, None
+
+
+ball_query = BallQuery.apply
 
 
 class GroupingOperation(Function):
@@ -91,3 +123,36 @@ class StackFarthestPointSampling(Function):
 
 
 stack_farthest_point_sample = StackFarthestPointSampling.apply
+
+
+class QueryAndGroup(nn.Module):
+    """ref :106-155"""
+
+    def __init__(self, radius: float, nsample: int, use_xyz: bool = True):
+        super().__init__()
+        self.radius, self.nsample, self.use_xyz = radius, nsample, use_xyz
+
+    def forward(self, xyz: torch.Tensor, xyz_batch_cnt: torch.Tensor, new_xyz: torch.Tensor,
+                new_xyz_batch_cnt: torch.Tensor, features: torch.Tensor = None):
+        """xyz (N1+N2..., 3), xyz_batch_cnt (B), new_xyz (M1+M2..., 3), new_xyz_batch_cnt (B), features (N1+N2..., C)
+        -> (new_features (M1+M2..., 3+C, nsample), idx (M1+M2..., nsample))"""
+        assert xyz.shape[0] == xyz_batch_cnt.sum(), 'xyz: %s, xyz_batch_cnt: %s' % (str(xyz.shape), str(new_xyz_batch_cnt))
+        assert new_xyz.shape[0] == new_xyz_batch_cnt.sum(), \
+            'new_xyz: %s, new_xyz_batch_cnt: %s' % (str(new_xyz.shape), str(new_xyz_batch_cnt))
+
+        idx, empty_ball_mask = ball_query(self.radius, self.nsample, xyz, xyz_batch_cnt, new_xyz, new_xyz_batch_cnt)
+        grouped_xyz = grouping_operation(xyz, xyz_batch_cnt, idx, new_xyz_batch_cnt)  # (M1+M2..., 3, nsample)
+        grouped_xyz -= new_xyz.unsqueeze(-1)
+        grouped_xyz[empty_ball_mask] = 0
+
+        if features is not None:
+            grouped_features = grouping_operation(features, xyz_batch_cnt, idx, new_xyz_batch_cnt)  # (M1+M2..., C, nsample)
+            grouped_features[empty_ball_mask] = 0
+            if self.use_xyz:
+                new_features = torch.cat([grouped_xyz, grouped_features], dim=1)  # (M1+M2..., 3+C, nsample)
+            else:
+                new_features = grouped_features
+        else:
+            assert self.use_xyz, "Cannot have not features and not use xyz as a feature!"
+            new_features = grouped_xyz
+        return new_features, idx
