@@ -27,7 +27,7 @@ BQ = [
     (2, 4096, 512, None, 0.8, 32, synth.cloud_ground_objects),
     (2, 4096, 512, None, 0.2, 16, synth.cloud_ground_objects),
     (2, 4096, 512, 0.4, 0.8, 32, synth.cloud_ground_objects),
-    (1, 1000, 333, None, 3.0, 8, synth.cloud_uniform),       # dense: early exit, n not a multiple of 4 (no TMA)
+    (1, 1000, 333, None, 3.0, 8, synth.cloud_uniform),       # dense: early exit, n not a multiple of 4
     (3, 1027, 70, 0.0, 1.5, 64, synth.cloud_dup_padded),      # ragged sizes, duplicates
     (2, 37, 5, None, 100.0, 7, synth.cloud_uniform),          # everything hits; nsample not a power of two
     (2, 2048, 130, None, 1e-3, 16, synth.cloud_uniform),      # nothing but the centre itself
@@ -35,14 +35,20 @@ BQ = [
     (2, 4096, 333, None, 0.8, 24, synth.cloud_ground_objects),    # half-warp kernel: two results per lane, odd centre count
     (2, 4096, 511, 0.2, 0.6, 17, synth.cloud_uniform),            # ... nsample just above 16, dilated
     (1, 2048, 100, None, 3.0, 32, synth.cloud_uniform),           # ... every super-round full of hits
+    (2, 300, 300, 0.1, 0.9, 40, synth.cloud_uniform),             # under 512 points: brute force only; dilated, nsample > 32
+    (1, 511, 511, None, 0.5, 33, synth.cloud_uniform),            # ... one point short of the grid
+    (4, 8192, 8192, None, 0.4, 16, synth.cloud_ground_objects),   # many centres per cloud (b * m = 32768)
+    (3, 4099, 2000, 0.3, 0.7, 64, synth.cloud_dup_padded),        # annulus through the merge kernel
+    (2, 1024, 1024, None, 2.0, 128, synth.cloud_uniform),         # rows four warps wide
+    (1, 4096, 2049, None, 0.8, 1, synth.cloud_ground_objects),    # nsample 1; one centre past a multiple of 128
 ]
 
 
-@pytest.mark.parametrize("algo", ["grid", "warp", "brute"])  # grid: half a warp per centre (nsample <= 32); warp: a whole one
+@pytest.mark.parametrize("algo", ["grid", "brute"])
 @pytest.mark.parametrize("case", BQ, ids=[f"bq{i}" for i in range(len(BQ))])
 def test_ball_query(orc, case, algo, monkeypatch):
     """Both query paths: the uniform-grid kernels (ball_query_grid.cu; clouds of >= 512 points whose grid is
-    usable) and the brute-force kernels (ball_query.cu), against the oracle."""
+    usable) and the brute-force kernel (ball_query.cu), against the oracle."""
     from tsmdet_b200 import pointnet2_utils as pu
 
     knob_setenv(monkeypatch, "TSMDET_BQ_ALGO", algo)
@@ -95,7 +101,7 @@ def test_ball_query_grid_edge_cases(orc):
 
 def test_ball_query_waymo_scale(orc):
     """BASELINE config 4 shape (65536 points, 16384 centres, r 0.8, ns 32): grid path vs the oracle on one
-    cloud, vs the brute-force kernels on all."""
+    cloud, vs the brute-force kernel on all."""
     import os
 
     from tsmdet_b200 import pointnet2_utils as pu

@@ -1,4 +1,4 @@
-// ball_query.cu -- radius / annulus neighbour query for sm_100a.
+// ball_query.cu -- radius / annulus neighbour query for sm_100a: the entry points and the brute-force search.
 //
 // Replaces (same idx / idx_cnt, bit for bit):
 //   ball_query_kernel_fast          /root/reference/pcdet/ops/pointnet2/pointnet2_batch/src/ball_query_gpu.cu:75-112
@@ -8,375 +8,144 @@
 // d2 < r^2 (dilated: rin^2 <= d2 < rout^2), idx_cnt = min(hits, nsample), the row is
 // padded cyclically with its own prefix, and a row without hits is all zeros.
 //
-// Design: one THREAD per centre; the cloud streams through shared memory in 1024-point tiles that
-// the TMA engine stages in their native (N,3) layout (cp.async.bulk, double buffered) and the CTA
-// re-packs into an x plane + a (y,z) plane.  Every lane of a warp tests the SAME point (a shared-memory
-// broadcast), so a hit appends to the thread's own row in index order with no atomics or ballots.
-// The inner loop is a conservative 1-D reject: d2 >= RN(dx*dx), so |dx| > r(1+2^-20) can never hit;
-// only points that survive it pay for the full reference distance (same FMA shape as the reference, so
-// the hit set is bit-identical).  For r = 0.2 m in a 70 m scene 99.4 % of the tests end after 4
-// instructions.
-#include <stdlib.h>
+// Design: clouds of a useful size are answered through a uniform grid (ball_query_grid.cu).  The brute-force search
+// below serves the rest -- clouds under 512 points, clouds whose grid is unusable, and TSMDET_BQ_ALGO=brute -- for the
+// batch query and for the stacked (ragged) one of stack_ball_query.cu: one warp per centre, lanes test 32 consecutive
+// points per step and append the hits in index order (ballot + popc).  Its kernels differ only in how a centre finds
+// its cloud and in the write-back; a cloud the grid answered (header word 9 set) is skipped.
 #include <string.h>
 
 #include "common.cuh"
+#include "grid.cuh"
 
 int tsm_ball_query_grid(bool dilated, int b, int n, int m, float rin, float rout, int nsample, const float* new_xyz,
                         const float* xyz, int* idx_cnt, int* idx, cudaStream_t stream, const int** grid_hdr);
 
 namespace tsm {
 
-constexpr int BQ_THREADS = 128;
-constexpr int BQ_TILE = 1024;  // points per shared-memory tile
+constexpr int BQ_WARPS = 8;
 
+// The first `nsample` hits, in index order, of the centre (cx, cy, cz) among the n points (N,3) of one cloud, written to
+// row[0..cnt) as index + off; returns cnt = min(hits, nsample) and the first hit's index in `first` (0 without hits).
 template <bool DILATED>
-__global__ void __launch_bounds__(BQ_THREADS)
-    ball_query_kernel(int n, int m, float rin2, float rout2, float rlim, int nsample,
-                      const float* __restrict__ new_xyz, const float* __restrict__ xyz, int* __restrict__ idx_cnt,
-                      int* __restrict__ idx, const int* __restrict__ perm, int* status,
-                      const int* __restrict__ grid_hdr) {
-    __shared__ __align__(128) float raw[2][BQ_TILE * 3];
-    __shared__ __align__(16) float sx[BQ_TILE];
-    __shared__ float2 syz[BQ_TILE];
-    __shared__ __align__(8) uint64_t full[2];
-
-    const int tid = threadIdx.x;
-    const int b = blockIdx.y;
-    if (grid_hdr && grid_hdr[b * 16 + 9]) return;  // answered by the grid query (ball_query_grid.cu)
-    xyz += (size_t)b * n * 3;
-    // Centres are handed out in x-sorted order (perm, built by sort_centres_kernel): the 32 centres of a
-    // warp then span a narrow x interval, so the per-lane reject below fails for (almost) all lanes at once
-    // and the warp skips the point without diverging.  Each thread still owns one output row.
-    const int slot = blockIdx.x * BQ_THREADS + tid;
-    const bool own = slot < m;
-    const int ci = own ? (perm ? perm[(size_t)b * m + slot] : slot) : 0;
-    const float* q = new_xyz + ((size_t)b * m + (own ? ci : 0)) * 3;
-    const float cx = q[0], cy = q[1], cz = q[2];
-    int* row = idx + ((size_t)b * m + (own ? ci : 0)) * nsample;
-    int cnt = own ? 0 : nsample;  // out-of-range threads are "full" from the start
-
-    const int ntiles = divup(n, BQ_TILE);
-    // TMA bulk copies need a 16-byte aligned source and size; otherwise plain loads.
-    const bool use_tma = ((reinterpret_cast<uintptr_t>(xyz) & 15) == 0) && ((n & 3) == 0);
-    if (use_tma && tid == 0) {
-        mbar_init(smem_u32(&full[0]), 1);
-        mbar_init(smem_u32(&full[1]), 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-
-    auto issue = [&](int t) {
-        const int start = t * BQ_TILE;
-        const int np = min(BQ_TILE, n - start);
-        const uint32_t bytes = (uint32_t)np * 12u;
-        mbar_arrive_expect_tx(smem_u32(&full[t & 1]), bytes);
-        bulk_g2s(smem_u32(&raw[t & 1][0]), xyz + (size_t)start * 3, bytes, smem_u32(&full[t & 1]));
-    };
-    if (use_tma && tid == 0) issue(0);
-
-    for (int t = 0; t < ntiles; ++t) {
-        const int start = t * BQ_TILE;
-        const int np = min(BQ_TILE, n - start);
-        if (use_tma) {
-            if (tid == 0 && t + 1 < ntiles) issue(t + 1);  // raw[(t+1)&1] was consumed by the re-pack of tile t-1
-            const uint32_t bar = smem_u32(&full[t & 1]);
-            const uint32_t ph = (uint32_t)((t >> 1) & 1);
-            if (!mbar_try_wait_cta(bar, ph)) {
-                const long long t0 = clock64();
-                while (!mbar_try_wait_cta(bar, ph))
-                    if (clock64() - t0 > 4000000000LL) watchdog_trip(status, TSM_ERR_WATCHDOG);
-            }
-            const float* rp = raw[t & 1];
-            for (int e = tid; e < np; e += BQ_THREADS) {  // stride-3 reads: conflict-free
-                sx[e] = rp[e * 3 + 0];
-                syz[e] = make_float2(rp[e * 3 + 1], rp[e * 3 + 2]);
-            }
-        } else {
-            for (int e = tid; e < np; e += BQ_THREADS) {
-                const float* p = xyz + (size_t)(start + e) * 3;
-                sx[e] = __ldg(p + 0);
-                syz[e] = make_float2(__ldg(p + 1), __ldg(p + 2));
-            }
+__device__ __forceinline__ int brute_query_core(int lane, int n, const float* __restrict__ pts, float cx, float cy,
+                                                float cz, float rin2, float rout2, int nsample, int* const row, int off,
+                                                int& first) {
+    int cnt = 0;
+    first = 0;
+    for (int base = 0; base < n && cnt < nsample; base += 32) {
+        const int k = base + lane;
+        bool hit = false;
+        if (k < n) {
+            const float d2 = sqdist3(__ldg(pts + 3 * k), __ldg(pts + 3 * k + 1), __ldg(pts + 3 * k + 2), cx, cy, cz);
+            hit = DILATED ? (d2 >= rin2 && d2 < rout2) : (d2 < rout2);
         }
-        __syncthreads();
-
-        if (cnt < nsample) {
-            auto full_test = [&](int k, float dx) {
-                const float2 yz = syz[k];
-                const float dy = __fsub_rn(cy, yz.x), dz = __fsub_rn(cz, yz.y);
-                const float d2 = __fmaf_rn(dz, dz, __fmaf_rn(dx, dx, __fmul_rn(dy, dy)));
-                const bool hit = DILATED ? (d2 >= rin2 && d2 < rout2) : (d2 < rout2);
-                if (hit && cnt < nsample) {
-                    row[cnt] = start + k;
-                    ++cnt;
-                }
-            };
-            int k = 0;
-            for (; k + 8 <= np; k += 8) {  // 8 points per step: two broadcast LDS.128, one branch
-                const float4 xa = *reinterpret_cast<const float4*>(&sx[k]);
-                const float4 xb = *reinterpret_cast<const float4*>(&sx[k + 4]);
-                const float d0 = __fsub_rn(cx, xa.x), d1 = __fsub_rn(cx, xa.y), d2_ = __fsub_rn(cx, xa.z),
-                            d3 = __fsub_rn(cx, xa.w), d4 = __fsub_rn(cx, xb.x), d5 = __fsub_rn(cx, xb.y),
-                            d6 = __fsub_rn(cx, xb.z), d7 = __fsub_rn(cx, xb.w);
-                const float mn = fminf(fminf(fminf(fabsf(d0), fabsf(d1)), fminf(fabsf(d2_), fabsf(d3))),
-                                       fminf(fminf(fabsf(d4), fabsf(d5)), fminf(fabsf(d6), fabsf(d7))));
-                if (mn < rlim) {
-                    if (fabsf(d0) < rlim) full_test(k + 0, d0);
-                    if (fabsf(d1) < rlim) full_test(k + 1, d1);
-                    if (fabsf(d2_) < rlim) full_test(k + 2, d2_);
-                    if (fabsf(d3) < rlim) full_test(k + 3, d3);
-                    if (fabsf(d4) < rlim) full_test(k + 4, d4);
-                    if (fabsf(d5) < rlim) full_test(k + 5, d5);
-                    if (fabsf(d6) < rlim) full_test(k + 6, d6);
-                    if (fabsf(d7) < rlim) full_test(k + 7, d7);
-                }
-            }
-            for (; k < np; ++k) {
-                const float dx = __fsub_rn(cx, sx[k]);
-                if (fabsf(dx) < rlim) full_test(k, dx);
-            }
-        }
-        // everyone is done with sx/syz (and raw[t&1]) before the next re-pack; stop once every row is full
-        if (__syncthreads_and(cnt >= nsample)) {
-            if (use_tma && t + 1 < ntiles) {  // drain the prefetch in flight before the CTA retires
-                const uint32_t bar = smem_u32(&full[(t + 1) & 1]);
-                const uint32_t ph = (uint32_t)(((t + 1) >> 1) & 1);
-                const long long t0 = clock64();
-                while (!mbar_try_wait_cta(bar, ph))
-                    if (clock64() - t0 > 4000000000LL) watchdog_trip(status, TSM_ERR_WATCHDOG);
-            }
-            break;
+        const unsigned bal = __ballot_sync(FULL, hit);
+        if (bal) {
+            if (cnt == 0) first = base + __ffs(bal) - 1;
+            const int pos = cnt + __popc(bal & ((1u << lane) - 1u));
+            if (hit && pos < nsample) row[pos] = k + off;
+            cnt += __popc(bal);
         }
     }
-
-    // ---- count + cyclic padding (row[p] = row[p mod cnt]); an empty row is zeroed
-    if (own) {
-        const int k = min(cnt, nsample);
-        idx_cnt[(size_t)b * m + ci] = k;
-        if (k == 0) {
-            for (int p = 0; p < nsample; ++p) row[p] = 0;
-        } else {
-            for (int p = k; p < nsample; ++p) row[p] = row[p - k];
-        }
-    }
+    return min(cnt, nsample);
 }
 
-// perm[b, :] = centre indices of cloud b sorted by x (bitonic sort in shared memory, m <= 8192).
-__global__ void __launch_bounds__(1024) sort_centres_kernel(int m, int mp2, const float* __restrict__ new_xyz,
-                                                            int* __restrict__ perm, const int* __restrict__ grid_hdr) {
-    extern __shared__ unsigned long long keys[];  // (ordered x bits << 32) | index; padding sorts last
-    const int b = blockIdx.x, tid = threadIdx.x;
-    if (grid_hdr && grid_hdr[b * 16 + 9]) return;  // answered by the grid query
-    for (int i = tid; i < mp2; i += 1024) {
-        unsigned long long k = ~0ull;
-        if (i < m) k = ((unsigned long long)f32_ordered(new_xyz[((size_t)b * m + i) * 3]) << 32) | (unsigned)i;
-        keys[i] = k;
-    }
-    __syncthreads();
-    for (int size = 2; size <= mp2; size <<= 1) {
-        for (int stride = size >> 1; stride > 0; stride >>= 1) {
-            for (int i = tid; i < (mp2 >> 1); i += 1024) {
-                const int lo = 2 * i - (i & (stride - 1));
-                const int hi = lo + stride;
-                const bool up = (lo & size) == 0;
-                const unsigned long long a = keys[lo], c = keys[hi];
-                if ((a > c) == up) {
-                    keys[lo] = c;
-                    keys[hi] = a;
-                }
-            }
-            __syncthreads();
-        }
-    }
-    for (int i = tid; i < m; i += 1024) perm[(size_t)b * m + i] = (int)(keys[i] & 0xffffffffu);
-}
-
-// ---- variant for FEW centres: one warp per group of 4 centres, lanes sweep 32 consecutive points per
-// step and compact hits in order with ballots (more parallelism per centre when B*M is small).
-constexpr int BQW_THREADS = 256;
-constexpr int BQW_WARPS = BQW_THREADS / 32;
-constexpr int BQW_CW = 4;          // centres per warp
-constexpr int BQW_TILE = 1024;     // points per shared-memory tile (12 KB)
-
+// Batch clouds (b, n, 3): CTA (x, cloud) holds BQ_WARPS warps that stride over the cloud's centres.
 template <bool DILATED>
-__global__ void __launch_bounds__(BQW_THREADS)
-    ball_query_warp_kernel(int n, int m, float rin2, float rout2, int nsample, const float* __restrict__ new_xyz,
-                      const float* __restrict__ xyz, int* __restrict__ idx_cnt, int* __restrict__ idx, int* status,
-                      const int* __restrict__ grid_hdr) {
-    __shared__ __align__(128) float tile[2][BQW_TILE * 3];
-    __shared__ __align__(8) uint64_t full[2];
-
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const int b = blockIdx.y;
-    if (grid_hdr && grid_hdr[b * 16 + 9]) return;  // answered by the grid query (ball_query_grid.cu)
-    xyz += (size_t)b * n * 3;
-    const int c0 = (blockIdx.x * BQW_WARPS + warp) * BQW_CW;  // first centre of this warp
-
-    float cx[BQW_CW], cy[BQW_CW], cz[BQW_CW];
-    int cnt[BQW_CW];
-#pragma unroll
-    for (int c = 0; c < BQW_CW; ++c) {
-        const int ci = c0 + c;
-        const bool ok = ci < m;
-        const float* q = new_xyz + ((size_t)b * m + (ok ? ci : 0)) * 3;
-        cx[c] = q[0];
-        cy[c] = q[1];
-        cz[c] = q[2];
-        cnt[c] = ok ? 0 : nsample;  // out-of-range centres are "full" from the start
-    }
-    int* rows = idx + ((size_t)b * m + c0) * nsample;
-
-    const int ntiles = divup(n, BQW_TILE);
-    // TMA bulk copies need 16-byte aligned source and size; otherwise plain loads.
-    const bool use_tma = ((reinterpret_cast<uintptr_t>(xyz) & 15) == 0) && ((n & 3) == 0);
-    if (use_tma && tid == 0) {
-        mbar_init(smem_u32(&full[0]), 1);
-        mbar_init(smem_u32(&full[1]), 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-
-    auto issue = [&](int t) {
-        const int start = t * BQW_TILE;
-        const int np = min(BQW_TILE, n - start);
-        const uint32_t bytes = (uint32_t)np * 12u;
-        mbar_arrive_expect_tx(smem_u32(&full[t & 1]), bytes);
-        bulk_g2s(smem_u32(&tile[t & 1][0]), xyz + (size_t)start * 3, bytes, smem_u32(&full[t & 1]));
-    };
-    if (use_tma && tid == 0) issue(0);
-
-    for (int t = 0; t < ntiles; ++t) {
-        const int start = t * BQW_TILE;
-        const int np = min(BQW_TILE, n - start);
-        const float* tp = tile[t & 1];
-        if (use_tma) {
-            if (tid == 0 && t + 1 < ntiles) issue(t + 1);  // buffer (t+1)&1 was released by the barrier below
-            const uint32_t bar = smem_u32(&full[t & 1]);
-            const uint32_t ph = (uint32_t)((t >> 1) & 1);
-            if (!mbar_try_wait_cta(bar, ph)) {
-                const long long t0 = clock64();
-                while (!mbar_try_wait_cta(bar, ph))
-                    if (clock64() - t0 > 4000000000LL) watchdog_trip(status, TSM_ERR_WATCHDOG);
-            }
-        } else {
-            for (int e = tid; e < np * 3; e += BQW_THREADS) tile[t & 1][e] = xyz[(size_t)start * 3 + e];
-            __syncthreads();
-        }
-
-        bool active = false;
-#pragma unroll
-        for (int c = 0; c < BQW_CW; ++c) active |= cnt[c] < nsample;
-        if (active) {
-            for (int base = 0; base < np; base += 32) {
-                const int pl = base + lane;
-                const bool valid = pl < np;
-                const float x = valid ? tp[pl * 3 + 0] : 0.f;
-                const float y = valid ? tp[pl * 3 + 1] : 0.f;
-                const float z = valid ? tp[pl * 3 + 2] : 0.f;
-#pragma unroll
-                for (int c = 0; c < BQW_CW; ++c) {
-                    if (cnt[c] < nsample) {  // warp-uniform
-                        const float d2 = sqdist3(x, y, z, cx[c], cy[c], cz[c]);
-                        const bool hit = valid && (DILATED ? (d2 >= rin2 && d2 < rout2) : (d2 < rout2));
-                        const unsigned bal = __ballot_sync(FULL, hit);
-                        if (bal) {
-                            const int pos = cnt[c] + __popc(bal & ((1u << lane) - 1u));
-                            if (hit && pos < nsample) rows[(size_t)c * nsample + pos] = start + pl;
-                            cnt[c] += __popc(bal);
-                        }
-                    }
-                }
-            }
-        }
-        // every warp must be done with tile[t&1] before it is refilled (tile t+2)
-        bool still = false;
-#pragma unroll
-        for (int c = 0; c < BQW_CW; ++c) still |= cnt[c] < nsample;
-        const int alldone = __syncthreads_and(!still);
-        if (alldone) {
-            if (use_tma && t + 1 < ntiles) {  // drain the prefetch in flight before the CTA retires
-                const uint32_t bar = smem_u32(&full[(t + 1) & 1]);
-                const uint32_t ph = (uint32_t)(((t + 1) >> 1) & 1);
-                const long long t0 = clock64();
-                while (!mbar_try_wait_cta(bar, ph))
-                    if (clock64() - t0 > 4000000000LL) watchdog_trip(status, TSM_ERR_WATCHDOG);
-            }
-            break;
-        }
-    }
-
-    // ---- counts + cyclic padding (row[p] = row[p mod cnt]); empty rows are zeroed
-    __syncwarp();
-#pragma unroll
-    for (int c = 0; c < BQW_CW; ++c) {
-        const int ci = c0 + c;
-        if (ci >= m) continue;
-        const int k = min(cnt[c], nsample);
-        int* row = rows + (size_t)c * nsample;
-        if (lane == 0) idx_cnt[(size_t)b * m + ci] = k;
-        if (k == 0) {
+__global__ void __launch_bounds__(BQ_WARPS * 32)
+    ball_query_brute_kernel(int n, int m, float rin2, float rout2, int nsample, const float* __restrict__ new_xyz,
+                            const float* __restrict__ xyz, const int* __restrict__ grid_hdr, int* __restrict__ idx_cnt,
+                            int* __restrict__ idx) {
+    const int lane = threadIdx.x & 31;
+    const int cloud = blockIdx.y;
+    if (grid_hdr && grid_hdr[cloud * kHdrInts + 9]) return;  // answered by the grid query
+    const float* const pts = xyz + (size_t)cloud * n * 3;
+    for (int c = blockIdx.x * BQ_WARPS + (threadIdx.x >> 5); c < m; c += gridDim.x * BQ_WARPS) {
+        const size_t wid = (size_t)cloud * m + c;
+        const float cx = __ldg(new_xyz + wid * 3), cy = __ldg(new_xyz + wid * 3 + 1), cz = __ldg(new_xyz + wid * 3 + 2);
+        int* const row = idx + wid * nsample;
+        int first;
+        const int cnt = brute_query_core<DILATED>(lane, n, pts, cx, cy, cz, rin2, rout2, nsample, row, 0, first);
+        // count + cyclic padding (row[p] = row[p mod cnt]); a row without hits is zeroed
+        __syncwarp();  // the prefix was written by whichever lanes owned it
+        if (lane == 0) idx_cnt[wid] = cnt;
+        if (cnt == 0) {
             for (int p = lane; p < nsample; p += 32) row[p] = 0;
-        } else if (k < nsample) {
-            for (int p = k + lane; p < nsample; p += 32) row[p] = row[p % k];
+        } else if (cnt < nsample) {
+            for (int p = cnt + lane; p < nsample; p += 32) row[p] = row[p % cnt];
         }
+    }
+}
+
+// Stacked (ragged) frames, one warp per centre, ball_query_kernel_stack's contract (bq_grid_query16_ragged_kernel in
+// ball_query_grid.cu spells it out): frame-local hits padded with the first one, only row[0] = -1 for an empty ball;
+// global_rows != 0: frame start + index, all-zero rows for empty balls.  idx_cnt may be null.
+__global__ void __launch_bounds__(BQ_WARPS * 32)
+    stack_ball_query_kernel(int b, int m, float r2, int nsample, const float* __restrict__ new_xyz,
+                            const int* __restrict__ mstart, const int* __restrict__ nstart,
+                            const float* __restrict__ xyz, const int* __restrict__ grid_hdr, int* __restrict__ idx_cnt,
+                            int* __restrict__ idx, int global_rows) {
+    const int lane = threadIdx.x & 31;
+    const int centre = blockIdx.x * BQ_WARPS + (threadIdx.x >> 5);
+    if (centre >= m) return;
+    const int f = stack_frame_of(centre, b, mstart);
+    if (grid_hdr && grid_hdr[f * kHdrInts + 9]) return;  // answered by the grid query
+    const int start = __ldg(nstart + f), n = __ldg(nstart + f + 1) - start;
+    const float cx = __ldg(new_xyz + (size_t)centre * 3), cy = __ldg(new_xyz + (size_t)centre * 3 + 1),
+                cz = __ldg(new_xyz + (size_t)centre * 3 + 2);
+    int* const row = idx + (size_t)centre * nsample;
+    const int off = global_rows ? start : 0;
+    int first;
+    const int cnt = brute_query_core<false>(lane, n, xyz + (size_t)start * 3, cx, cy, cz, 0.f, r2, nsample, row, off,
+                                            first);
+    if (idx_cnt && lane == 0) idx_cnt[centre] = cnt;
+    if (cnt == 0) {
+        if (global_rows)
+            for (int p = lane; p < nsample; p += 32) row[p] = 0;
+        else if (lane == 0)
+            row[0] = -1;
+    } else {
+        for (int p = cnt + lane; p < nsample; p += 32) row[p] = first + off;
     }
 }
 
 }  // namespace tsm
 
+int tsm_stack_ball_query_brute(int b, int m, float radius, int nsample, const float* new_xyz, const int* mstart,
+                               const int* nstart, const float* xyz, const int* grid_hdr, int* idx, int* idx_cnt,
+                               int global_rows, cudaStream_t stream) {
+    using namespace tsm;
+    stack_ball_query_kernel<<<(unsigned)divup(m, BQ_WARPS), BQ_WARPS * 32, 0, stream>>>(
+        b, m, radius * radius, nsample, new_xyz, mstart, nstart, xyz, grid_hdr, idx_cnt, idx, global_rows);
+    TSM_LAUNCH_CHECK();
+    return TSM_OK;
+}
+
 static int run_ball_query(bool dilated, int b, int n, int m, float rin, float rout, int nsample, const float* new_xyz,
                           const float* xyz, int* idx_cnt, int* idx, cudaStream_t stream) {
+    using namespace tsm;
     if (b <= 0 || m <= 0) return TSM_OK;
     if (n < 0 || nsample <= 0 || b > 65535) return TSM_ERR_INVALID;
     const float rin2 = rin * rin;    // f32 products, as ball_query_gpu.cu:91, 154-155
     const float rout2 = rout * rout;
-    // conservative reject bound: any |dx| above it has RN(dx*dx) >= rout2 (NaN/inf radii disable it)
-    float rlim = fabsf(rout) * 1.000002f + 1e-30f;
-    if (!(rlim < 3.0e38f)) rlim = 3.4e38f;
-    int* status = tsm_status_word(stream);
-    // Clouds of a useful size are answered through a uniform grid (ball_query_grid.cu): ~100x fewer distance
-    // tests than the brute-force kernels below, which then only serve the clouds whose grid was unusable
-    // (flagged on the device; they exit at once for the others).  TSMDET_BQ_ALGO=brute disables the grid.
+    // The grid query answers every cloud whose grid is usable and flags it on the device; the brute-force kernel then
+    // exits at once for those clouds (no host synchronisation either way).  TSMDET_BQ_ALGO=brute disables the grid.
     const int* ghdr = nullptr;
-    {
-        const char* algo = tsm_knob(KNOB_BQ_ALGO);
-        if (n >= 512 && !(algo && !strcmp(algo, "brute"))) {
-            const int rc = tsm_ball_query_grid(dilated, b, n, m, rin, rout, nsample, new_xyz, xyz, idx_cnt, idx, stream,
-                                               &ghdr);
-            if (rc != TSM_OK) return rc;
-        }
+    const char* algo = tsm_knob(KNOB_BQ_ALGO);
+    if (n >= 512 && !(algo && !strcmp(algo, "brute"))) {
+        const int rc = tsm_ball_query_grid(dilated, b, n, m, rin, rout, nsample, new_xyz, xyz, idx_cnt, idx, stream,
+                                           &ghdr);
+        if (rc != TSM_OK) return rc;
     }
-    if ((long)b * m >= 32768) {  // enough centres to fill the GPU with one thread each
-        int* perm = nullptr;
-        if (m <= 8192 && m >= 64) {
-            void* p = nullptr;
-            int rc = tsm_scratch_get(3, sizeof(int) * (size_t)b * m, stream, &p);
-            if (rc != TSM_OK) return rc;
-            perm = (int*)p;
-            int mp2 = 64;
-            while (mp2 < m) mp2 <<= 1;
-            const size_t dyn = sizeof(unsigned long long) * (size_t)mp2;
-            if (dyn > 48 * 1024)
-                TSM_CUDA_TRY(cudaFuncSetAttribute(tsm::sort_centres_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
-            tsm::sort_centres_kernel<<<b, 1024, dyn, stream>>>(m, mp2, new_xyz, perm, ghdr);
-            TSM_LAUNCH_CHECK();
-        }
-        dim3 grid((unsigned)tsm::divup(m, tsm::BQ_THREADS), (unsigned)b);
-        if (dilated)
-            tsm::ball_query_kernel<true><<<grid, tsm::BQ_THREADS, 0, stream>>>(n, m, rin2, rout2, rlim, nsample, new_xyz,
-                                                                                xyz, idx_cnt, idx, perm, status, ghdr);
-        else
-            tsm::ball_query_kernel<false><<<grid, tsm::BQ_THREADS, 0, stream>>>(n, m, rin2, rout2, rlim, nsample,
-                                                                                 new_xyz, xyz, idx_cnt, idx, perm, status, ghdr);
-    } else {
-        dim3 grid((unsigned)tsm::divup(m, tsm::BQW_WARPS * tsm::BQW_CW), (unsigned)b);
-        if (dilated)
-            tsm::ball_query_warp_kernel<true><<<grid, tsm::BQW_THREADS, 0, stream>>>(n, m, rin2, rout2, nsample, new_xyz,
-                                                                                     xyz, idx_cnt, idx, status, ghdr);
-        else
-            tsm::ball_query_warp_kernel<false><<<grid, tsm::BQW_THREADS, 0, stream>>>(n, m, rin2, rout2, nsample,
-                                                                                      new_xyz, xyz, idx_cnt, idx, status, ghdr);
-    }
+    // 16 centres per warp: a CTA for every 128 centres keeps the launch small where the grid answered every cloud
+    const dim3 grid((unsigned)divup(m, BQ_WARPS * 16), (unsigned)b);
+    if (dilated)
+        ball_query_brute_kernel<true><<<grid, BQ_WARPS * 32, 0, stream>>>(n, m, rin2, rout2, nsample, new_xyz, xyz, ghdr,
+                                                                          idx_cnt, idx);
+    else
+        ball_query_brute_kernel<false><<<grid, BQ_WARPS * 32, 0, stream>>>(n, m, rin2, rout2, nsample, new_xyz, xyz, ghdr,
+                                                                           idx_cnt, idx);
     TSM_LAUNCH_CHECK();
     return TSM_OK;
 }

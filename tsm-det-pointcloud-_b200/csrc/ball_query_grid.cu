@@ -10,22 +10,21 @@
 //    (histogram, scan, scatter) -> a per-cell fix-up that puts every cell's points in ASCENDING ORIGINAL
 //    INDEX (each point counts the members of its cell with a smaller index).  Output: cell_start[] and
 //    the points as (x, y, z, index) float4 records in cell order.
-//  * bq_grid_query_kernel (nsample <= 32), one warp per centre, candidate-parallel: see the kernel.
+//  * bq_grid_query16_kernel (nsample <= 32), half a warp per centre, candidate-parallel: see grid_query16_core.
 //  * bq_grid_merge_kernel (larger nsample), one warp per centre: lane l < 27 walks the sorted list of one
 //    neighbour cell up to its next hit; the warp repeatedly takes the smallest pending index
 //    (redux.sync.min) until `nsample` are out.
 //    Both evaluate the reference's own distance expression, so the hit set is identical.
 //
 // A cloud whose points pile up in one cell (> kMaxCell per cell: degenerate input, or r comparable to the
-// whole cloud) is flagged and left to the brute-force kernels of ball_query.cu, which skip flagged-OK
+// whole cloud) is flagged and left to the brute-force search of ball_query.cu, which skips flagged-OK
 // clouds -- no host synchronisation either way.
 //
 // Stacked (ragged) frames, pointnet2_stack's ball query: bq_grid_build_ragged_kernel builds one grid per frame over its
 // own points and bq_grid_query16_ragged_kernel / bq_grid_merge_ragged_kernel run the same search cores
 // (grid_query16_core, grid_merge_core); they differ only in finding the centre's frame and in the write-back (first-hit
-// padding, -1 for an empty ball).  Unusable frames go to stack_ball_query_brute_kernel (stack_ball_query.cu).
+// padding, -1 for an empty ball).  Unusable frames go to stack_ball_query_kernel (ball_query.cu).
 #include <math.h>
-#include <string.h>
 
 #include "common.cuh"
 #include "grid.cuh"
@@ -290,100 +289,13 @@ __global__ void __launch_bounds__(256)
     }
 }
 
-// ns <= 32: CANDIDATE-parallel.  The candidates of the 27 cells are numbered 0..C-1 (prefix sum over the lanes'
-// cell populations); in super-rounds of 128 every lane loads four of them at once (independent loads: one
-// L2 round trip per 128 candidates instead of one per emitted hit), keeps the hits, and the warp extracts the
-// smallest pending indices with redux.sync.min.  Lane e ends up holding the e-th smallest hit; it re-enters
-// the next super-round as a fifth pending value, so the result is the nsample smallest indices overall.
-template <bool DILATED>
-__global__ void __launch_bounds__(256)
-    bq_grid_query_kernel(int b, int n, int m, float rin2, float rout2, int nsample, const float* __restrict__ new_xyz,
-                         const int* __restrict__ hdr_all, const int* __restrict__ cell_start_all,
-                         const float4* __restrict__ sorted_all, int* __restrict__ idx_cnt, int* __restrict__ idx) {
-    constexpr int K = 4;
-    constexpr uint32_t NONE = 0xffffffffu;
-    const int lane = threadIdx.x & 31;
-    const long long wid = (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-    if (wid >= (long long)b * m) return;
-    const int cloud = (int)(wid / m);
-    const GridHdr h = *reinterpret_cast<const GridHdr*>(hdr_all + (size_t)cloud * kHdrInts);
-    if (!h.ok) return;
-    const int* __restrict__ cell_start = cell_start_all + (size_t)cloud * (kGridCells + 1);
-    const float4* __restrict__ sorted = sorted_all + (size_t)cloud * n;
-    const float* q = new_xyz + (size_t)wid * 3;
-    const float cx = __ldg(q), cy = __ldg(q + 1), cz = __ldg(q + 2);
-    int* const row = idx + (size_t)wid * nsample;
-
-    int beg = 0, len = 0;
-    if (lane < 27) {
-        const int gx = grid_q(cx, h.lo[0], h.inv[0], h.n[0]) + lane % 3 - 1;
-        const int gy = grid_q(cy, h.lo[1], h.inv[1], h.n[1]) + (lane / 3) % 3 - 1;
-        const int gz = grid_q(cz, h.lo[2], h.inv[2], h.n[2]) + lane / 9 - 1;
-        if (gx >= 0 && gx < h.n[0] && gy >= 0 && gy < h.n[1] && gz >= 0 && gz < h.n[2]) {
-            const int c = (gz * h.n[1] + gy) * h.n[0] + gx;
-            beg = __ldg(cell_start + c);
-            len = __ldg(cell_start + c + 1) - beg;
-        }
-    }
-    int incl = len;  // inclusive prefix of the cell populations
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        const int t = __shfl_up_sync(FULL, incl, o);
-        if (lane >= o) incl += t;
-    }
-    const int total = __shfl_sync(FULL, incl, 31);
-    const int excl_beg = beg - (incl - len);  // candidate j of this lane's cell sits at sorted[excl_beg + j]
-
-    uint32_t best = NONE;  // lane e: the e-th smallest hit so far
-    for (int base = 0; base < total; base += 32 * K) {
-        uint32_t v[K + 1];
-#pragma unroll
-        for (int k = 0; k < K; ++k) {
-            v[k] = NONE;
-            if (base + k * 32 >= total) continue;  // (uniform) no candidates left for this slot: skip the search
-            const int j = base + k * 32 + lane;
-            // owner cell = first lane whose inclusive prefix exceeds j (binary search over the lanes)
-            int t = 0;
-#pragma unroll
-            for (int step = 16; step > 0; step >>= 1) {
-                const int val = __shfl_sync(FULL, incl, t + step - 1);
-                if (val <= j) t += step;
-            }
-            const int src = __shfl_sync(FULL, excl_beg, t & 31) + j;
-            if (j < total) {
-                const float4 p = sorted[src];
-                const float d2 = sqdist3(p.x, p.y, p.z, cx, cy, cz);
-                const bool hit = DILATED ? (d2 >= rin2 && d2 < rout2) : (d2 < rout2);
-                if (hit) v[k] = (uint32_t)__float_as_int(p.w);
-            }
-        }
-        v[K] = best;
-        uint32_t nb = NONE;
-        for (int e = 0; e < nsample; ++e) {
-            uint32_t mine = v[0];
-#pragma unroll
-            for (int k = 1; k <= K; ++k) mine = min(mine, v[k]);
-            const uint32_t mn = __reduce_min_sync(FULL, mine);
-            if (mn == NONE) break;
-#pragma unroll
-            for (int k = 0; k <= K; ++k)
-                if (v[k] == mn) v[k] = NONE;  // indices are unique: exactly one slot in the warp
-            if (lane == e) nb = mn;
-        }
-        best = nb;
-    }
-    const int cnt = __popc(__ballot_sync(FULL, best != NONE));
-    if (lane == 0) idx_cnt[wid] = cnt;
-    // row[p] = hit[p mod cnt] (cyclic padding); rows without hits are zeroed
-    for (int p = lane; p < nsample; p += 32) {
-        const uint32_t val = __shfl_sync(FULL, best, cnt ? p % cnt : 0);
-        row[p] = cnt ? (int)val : 0;
-    }
-}
-
 // The half-warp search of bq_grid_query16_kernel for the centre (cx, cy, cz) in one cloud's grid: lane e of the half
 // ends with the (e + 16 i)-th smallest hit index in best[i] (NONE past the last); returns the number of hits kept
-// (<= nsample).
+// (<= nsample).  CANDIDATE-parallel: the candidates of the 27 cells are numbered 0..C-1 (prefix sum over the lanes' cell
+// populations); in super-rounds of 64 every lane loads four of them at once (independent loads: one L2 round trip per
+// 64 candidates instead of one per emitted hit), keeps the hits, and the half-warp extracts the smallest pending indices
+// with redux.sync.min.  The kept hits re-enter the next super-round as pending values, so the result is the nsample
+// smallest indices overall.
 template <bool DILATED, int R>
 __device__ __forceinline__ int grid_query16_core(int gl, unsigned gmask, const GridHdr& h, const int* __restrict__ cell_start,
                                                  const float4* __restrict__ sorted, float cx, float cy, float cz, float rin2,
@@ -468,7 +380,7 @@ __device__ __forceinline__ int grid_query16_core(int gl, unsigned gmask, const G
     return cnt;
 }
 
-// nsample <= 16 * R (R = 1, 2): the same algorithm with HALF a warp per centre (two centres per warp).  At the first SA layer a ball
+// nsample <= 16 * R (R = 1, 2): HALF a warp per centre (two centres per warp).  At the first SA layer a ball
 // holds one or two points (the centre itself and maybe a neighbour) and a few dozen candidates, so a whole warp per centre
 // is mostly fixed cost: ncu counts 346 warp-instructions per centre at 80 % issue utilisation -- the kernel is
 // instruction-bound.  A lane owns neighbour cells gl and gl + 16 (candidates may be numbered in any order: the result is
@@ -515,7 +427,7 @@ __global__ void __launch_bounds__(256)
 // stack_frame_of(p); its row holds the first min(hits, nsample) frame-local hit indices in ascending order, the
 // remaining slots repeat the FIRST hit, and a row without hits gets only row[0] = -1 (the caller zeroed the rest).
 // global_rows != 0 (the fused SA path): frame start + index instead, and all-zero rows without hits.  idx_cnt may be
-// null.  Frames whose grid is unusable are left to stack_ball_query_brute_kernel (stack_ball_query.cu).
+// null.  Frames whose grid is unusable are left to stack_ball_query_kernel (ball_query.cu).
 template <int R>
 __global__ void __launch_bounds__(256)
     bq_grid_query16_ragged_kernel(int b, int m, float rout2, int nsample, const float* __restrict__ new_xyz,
@@ -591,50 +503,65 @@ __global__ void __launch_bounds__(256)
     }
 }
 
+constexpr int kBuildSmem = kGridCells * sizeof(uint32_t);  // the build's shared-memory histogram
+
+// The grids of b clouds holding npts points in all, carved from scratch buffer `tag`: the headers, the cell starts and
+// the scattered / index-sorted point records, each array 256-byte aligned.
+struct GridScratch {
+    int* hdr;
+    int* cell_start;
+    float4* tmp;
+    float4* sorted;
+};
+
+static int grid_scratch(int tag, int b, size_t npts, cudaStream_t stream, GridScratch* g) {
+    auto align = [](size_t bytes) { return (bytes + 255) & ~(size_t)255; };
+    const size_t hdr_bytes = align((size_t)b * kHdrInts * sizeof(int));
+    const size_t cs_bytes = align((size_t)b * (kGridCells + 1) * sizeof(int));
+    const size_t pts_bytes = align(npts * sizeof(float4));
+    void* base = nullptr;
+    const int rc = tsm_scratch_get(tag, hdr_bytes + cs_bytes + 2 * pts_bytes, stream, &base);
+    if (rc != TSM_OK) return rc;
+    unsigned char* const p = static_cast<unsigned char*>(base);
+    g->hdr = reinterpret_cast<int*>(p);
+    g->cell_start = reinterpret_cast<int*>(p + hdr_bytes);
+    g->tmp = reinterpret_cast<float4*>(p + hdr_bytes + cs_bytes);
+    g->sorted = reinterpret_cast<float4*>(p + hdr_bytes + cs_bytes + pts_bytes);
+    return TSM_OK;
+}
+
 }  // namespace tsm
 
 int tsm_grid_build(int b, int n, float rout, const float* xyz, cudaStream_t stream, int tag, const int** hdr_out,
                    const int** cell_start_out, const float4** sorted_out) {
     using namespace tsm;
-    const size_t hdr_bytes = ((size_t)b * kHdrInts * sizeof(int) + 255) & ~(size_t)255;
-    const size_t cs_bytes = ((size_t)b * (kGridCells + 1) * sizeof(int) + 255) & ~(size_t)255;
-    const size_t pts_bytes = ((size_t)b * n * sizeof(float4) + 255) & ~(size_t)255;
-    void* base = nullptr;
-    int rc = tsm_scratch_get(tag, hdr_bytes + cs_bytes + 2 * pts_bytes, stream, &base);
+    GridScratch g;
+    const int rc = grid_scratch(tag, b, (size_t)b * n, stream, &g);
     if (rc != TSM_OK) return rc;
-    unsigned char* p = static_cast<unsigned char*>(base);
-    int* hdr = reinterpret_cast<int*>(p);
-    int* cell_start = reinterpret_cast<int*>(p + hdr_bytes);
-    float4* tmp = reinterpret_cast<float4*>(p + hdr_bytes + cs_bytes);
-    float4* sorted = reinterpret_cast<float4*>(p + hdr_bytes + cs_bytes + pts_bytes);
-    const size_t dyn = (size_t)kGridCells * sizeof(uint32_t);
-    TSM_CUDA_TRY(cudaFuncSetAttribute(bq_grid_build_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
-    bq_grid_build_kernel<<<b, 1024, dyn, stream>>>(n, rout, xyz, hdr, cell_start, tmp, sorted);
+    TSM_CUDA_TRY(cudaFuncSetAttribute(bq_grid_build_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kBuildSmem));
+    bq_grid_build_kernel<<<b, 1024, kBuildSmem, stream>>>(n, rout, xyz, g.hdr, g.cell_start, g.tmp, g.sorted);
     TSM_LAUNCH_CHECK();
-    *hdr_out = hdr;
-    *cell_start_out = cell_start;
-    *sorted_out = sorted;
+    *hdr_out = g.hdr;
+    *cell_start_out = g.cell_start;
+    *sorted_out = g.sorted;
     return TSM_OK;
 }
 
 // Builds the grids of all clouds and answers every cloud whose grid is usable.  *grid_hdr receives the
-// per-cloud header array (device; int [b][16], word 9 = usable) for the brute-force kernels to consult.
+// per-cloud header array (device; int [b][16], word 9 = usable) for the brute-force kernel to consult.
 int tsm_ball_query_grid(bool dilated, int b, int n, int m, float rin, float rout, int nsample, const float* new_xyz,
                         const float* xyz, int* idx_cnt, int* idx, cudaStream_t stream, const int** grid_hdr) {
     using namespace tsm;
     const int *hdr = nullptr, *cell_start = nullptr;
     const float4* sorted = nullptr;
-    if (!(rout > 0.f)) {  // no ball: nothing can hit; leave every cloud to the brute-force kernels
+    if (!(rout > 0.f)) {  // no ball: nothing can hit; leave every cloud to the brute-force kernel
         *grid_hdr = nullptr;
         return TSM_OK;
     }
     int rc = tsm_grid_build(b, n, rout, xyz, stream, 4, &hdr, &cell_start, &sorted);
     if (rc != TSM_OK) return rc;
     const float rin2 = rin * rin, rout2 = rout * rout;  // f32 products, as ball_query_gpu.cu:91, 154-155
-    const long long warps = (long long)b * m;
-    const unsigned blocks = (unsigned)((warps + 7) / 8);
-    const char* bq_full = tsm_knob(KNOB_BQ_ALGO);  // "warp": a whole warp per centre (A/B, tests)
-    if (nsample <= 32 && kMaxCell * 27 < 32768 && !(bq_full && !strcmp(bq_full, "warp"))) {
+    if (nsample <= 32) {
         const dim3 grid16((unsigned)((m + 15) / 16), (unsigned)b);
 #define BQ16(D, RR) bq_grid_query16_kernel<D, RR><<<grid16, 256, 0, stream>>>(n, m, rin2, rout2, nsample, new_xyz, hdr, cell_start, sorted, idx_cnt, idx)
         if (nsample <= 16) {
@@ -643,14 +570,8 @@ int tsm_ball_query_grid(bool dilated, int b, int n, int m, float rin, float rout
             if (dilated) BQ16(true, 2); else BQ16(false, 2);
         }
 #undef BQ16
-    } else if (nsample <= 32) {
-        if (dilated)
-            bq_grid_query_kernel<true><<<blocks, 256, 0, stream>>>(b, n, m, rin2, rout2, nsample, new_xyz, hdr,
-                                                                   cell_start, sorted, idx_cnt, idx);
-        else
-            bq_grid_query_kernel<false><<<blocks, 256, 0, stream>>>(b, n, m, rin2, rout2, nsample, new_xyz, hdr,
-                                                                    cell_start, sorted, idx_cnt, idx);
     } else {
+        const unsigned blocks = (unsigned)(((long long)b * m + 7) / 8);
         if (dilated)
             bq_grid_merge_kernel<true><<<blocks, 256, 0, stream>>>(b, n, m, rin2, rout2, nsample, new_xyz, hdr,
                                                                    cell_start, sorted, idx_cnt, idx);
@@ -672,36 +593,27 @@ int tsm_stack_ball_query_grid(int b, int m, int n_total, float radius, int nsamp
     // frame then goes to the brute-force kernel)
     const float rout = fabsf(radius);
     if (!(rout > 0.f) || n_total <= 0) return TSM_OK;
-    const size_t hdr_bytes = ((size_t)b * kHdrInts * sizeof(int) + 255) & ~(size_t)255;
-    const size_t cs_bytes = ((size_t)b * (kGridCells + 1) * sizeof(int) + 255) & ~(size_t)255;
-    const size_t pts_bytes = ((size_t)n_total * sizeof(float4) + 255) & ~(size_t)255;
-    void* base = nullptr;
-    int rc = tsm_scratch_get(9, hdr_bytes + cs_bytes + 2 * pts_bytes, stream, &base);
+    GridScratch g;
+    const int rc = grid_scratch(9, b, (size_t)n_total, stream, &g);
     if (rc != TSM_OK) return rc;
-    unsigned char* p = static_cast<unsigned char*>(base);
-    int* hdr = reinterpret_cast<int*>(p);
-    int* cell_start = reinterpret_cast<int*>(p + hdr_bytes);
-    float4* tmp = reinterpret_cast<float4*>(p + hdr_bytes + cs_bytes);
-    float4* sorted = reinterpret_cast<float4*>(p + hdr_bytes + cs_bytes + pts_bytes);
-    const size_t dyn = (size_t)kGridCells * sizeof(uint32_t);
-    TSM_CUDA_TRY(cudaFuncSetAttribute(bq_grid_build_ragged_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
-    bq_grid_build_ragged_kernel<<<b, 1024, dyn, stream>>>(rout, nstart, xyz, hdr, cell_start, tmp, sorted);
+    TSM_CUDA_TRY(cudaFuncSetAttribute(bq_grid_build_ragged_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kBuildSmem));
+    bq_grid_build_ragged_kernel<<<b, 1024, kBuildSmem, stream>>>(rout, nstart, xyz, g.hdr, g.cell_start, g.tmp, g.sorted);
     TSM_LAUNCH_CHECK();
     const float rout2 = radius * radius;  // f32 product, as ball_query_gpu.cu (stack):25
     if (nsample <= 32) {
         const unsigned blocks = (unsigned)((m + 15) / 16);
         if (nsample <= 16)
-            bq_grid_query16_ragged_kernel<1><<<blocks, 256, 0, stream>>>(b, m, rout2, nsample, new_xyz, mstart, nstart, hdr,
-                                                                         cell_start, sorted, idx_cnt, idx, global_rows);
+            bq_grid_query16_ragged_kernel<1><<<blocks, 256, 0, stream>>>(b, m, rout2, nsample, new_xyz, mstart, nstart, g.hdr,
+                                                                         g.cell_start, g.sorted, idx_cnt, idx, global_rows);
         else
-            bq_grid_query16_ragged_kernel<2><<<blocks, 256, 0, stream>>>(b, m, rout2, nsample, new_xyz, mstart, nstart, hdr,
-                                                                         cell_start, sorted, idx_cnt, idx, global_rows);
+            bq_grid_query16_ragged_kernel<2><<<blocks, 256, 0, stream>>>(b, m, rout2, nsample, new_xyz, mstart, nstart, g.hdr,
+                                                                         g.cell_start, g.sorted, idx_cnt, idx, global_rows);
     } else {
         bq_grid_merge_ragged_kernel<<<(unsigned)((m + 7) / 8), 256, 0, stream>>>(b, m, rout2, nsample, new_xyz, mstart, nstart,
-                                                                                 hdr, cell_start, sorted, idx_cnt, idx,
+                                                                                 g.hdr, g.cell_start, g.sorted, idx_cnt, idx,
                                                                                  global_rows);
     }
     TSM_LAUNCH_CHECK();
-    *grid_hdr = hdr;
+    *grid_hdr = g.hdr;
     return TSM_OK;
 }

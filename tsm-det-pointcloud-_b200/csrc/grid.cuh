@@ -44,3 +44,9 @@ int tsm_grid_build(int b, int n, float rout, const float* xyz, cudaStream_t stre
 int tsm_stack_ball_query_grid(int b, int m, int n_total, float radius, int nsample, const float* new_xyz,
                               const int* mstart, const int* nstart, const float* xyz, int* idx, int* idx_cnt,
                               int global_rows, cudaStream_t stream, const int** grid_hdr);
+
+// Stacked clouds by brute force (ball_query.cu): every centre of a frame whose header word 9 is not set (all of them when
+// grid_hdr is nullptr), same arguments and contract as the grid query.
+int tsm_stack_ball_query_brute(int b, int m, float radius, int nsample, const float* new_xyz, const int* mstart,
+                               const int* nstart, const float* xyz, const int* grid_hdr, int* idx, int* idx_cnt,
+                               int global_rows, cudaStream_t stream);

@@ -12,8 +12,8 @@
 // Design: the frame starts come from a device-side scan of the two count arrays (no host synchronisation); every frame
 // then gets its own uniform grid over its own points (bq_grid_build_ragged_kernel, the same build as the batch grid
 // query, ball_query_grid.cu) and is answered by the half-warp / merge grid queries.  Frames whose grid is unusable
-// (> kMaxCell points in one cell, a non-finite extent, no points) and TSMDET_BQ_ALGO=brute go to
-// stack_ball_query_brute_kernel below, which skips the frames the grid answered.
+// (> kMaxCell points in one cell, a non-finite extent, no points) and TSMDET_BQ_ALGO=brute go to the brute-force
+// search of ball_query.cu (stack_ball_query_kernel), which skips the frames the grid answered.
 #include <string.h>
 
 #include <algorithm>
@@ -46,54 +46,6 @@ __global__ void __launch_bounds__(64) stack_counts_scan_kernel(int b, const int*
         carry += __shfl_sync(FULL, inc, 31);
     }
     if (lane == 0) out[b] = carry;
-}
-
-// One warp per centre: lanes test 32 consecutive points of the frame per step and append the hits in index order
-// (ballot + popc).  Frames answered by the grid query (grid_hdr word 9) are skipped.
-constexpr int SBQ_WARPS = 8;
-
-__global__ void __launch_bounds__(SBQ_WARPS * 32)
-    stack_ball_query_brute_kernel(int b, int m, float r2, int nsample, const float* __restrict__ new_xyz,
-                                  const int* __restrict__ mstart, const int* __restrict__ nstart,
-                                  const float* __restrict__ xyz, const int* __restrict__ grid_hdr,
-                                  int* __restrict__ idx_cnt, int* __restrict__ idx, int global_rows) {
-    const int lane = threadIdx.x & 31;
-    const int centre = blockIdx.x * SBQ_WARPS + (threadIdx.x >> 5);
-    if (centre >= m) return;
-    const int f = stack_frame_of(centre, b, mstart);
-    if (grid_hdr && grid_hdr[f * kHdrInts + 9]) return;  // answered by the grid query
-    const int start = __ldg(nstart + f), n = __ldg(nstart + f + 1) - start;
-    const float* const pts = xyz + (size_t)start * 3;
-    const float cx = __ldg(new_xyz + (size_t)centre * 3), cy = __ldg(new_xyz + (size_t)centre * 3 + 1),
-                cz = __ldg(new_xyz + (size_t)centre * 3 + 2);
-    int* const row = idx + (size_t)centre * nsample;
-    const int off = global_rows ? start : 0;
-    int cnt = 0, first = 0;
-    for (int base = 0; base < n && cnt < nsample; base += 32) {
-        const int k = base + lane;
-        bool hit = false;
-        if (k < n) {
-            const float d2 = sqdist3(__ldg(pts + 3 * k), __ldg(pts + 3 * k + 1), __ldg(pts + 3 * k + 2), cx, cy, cz);
-            hit = d2 < r2;
-        }
-        const unsigned bal = __ballot_sync(FULL, hit);
-        if (bal) {
-            if (cnt == 0) first = base + __ffs(bal) - 1;
-            const int pos = cnt + __popc(bal & ((1u << lane) - 1u));
-            if (hit && pos < nsample) row[pos] = k + off;
-            cnt += __popc(bal);
-        }
-    }
-    cnt = min(cnt, nsample);
-    if (idx_cnt && lane == 0) idx_cnt[centre] = cnt;
-    if (cnt == 0) {
-        if (global_rows)
-            for (int p = lane; p < nsample; p += 32) row[p] = 0;
-        else if (lane == 0)
-            row[0] = -1;
-    } else {
-        for (int p = cnt + lane; p < nsample; p += 32) row[p] = first + off;
-    }
 }
 
 // Stacked features (N,C) fp32 -> rows (N,Cp) in the fused MLP's operand type, zero padded, rounded exactly as
@@ -148,10 +100,8 @@ int tsmdet_stack_ball_query(int b, int m, int n_total, float radius, int nsample
                                        global_rows, stream, &ghdr);
         if (rc != TSM_OK) return rc;
     }
-    stack_ball_query_brute_kernel<<<(unsigned)divup(m, SBQ_WARPS), SBQ_WARPS * 32, 0, stream>>>(
-        b, m, radius * radius, nsample, new_xyz, mstart, nstart, xyz, ghdr, idx_cnt, idx, global_rows);
-    TSM_LAUNCH_CHECK();
-    return TSM_OK;
+    return tsm_stack_ball_query_brute(b, m, radius, nsample, new_xyz, mstart, nstart, xyz, ghdr, idx, idx_cnt, global_rows,
+                                      stream);
 }
 
 int tsmdet_stack_feature_rows(int precision, int n, int c, const float* features, void* rows, void* stream) {
