@@ -245,6 +245,21 @@ int tsmdet_stack_ball_query(int b, int m, int n_total, float radius, int nsample
  * the rounding the kernels apply to (B,C,N) planes themselves.  Pass the result as features_t of
  * tsmdet_sa_mlp_maxpool_packed_p with B = 1. */
 int tsmdet_stack_feature_rows(int precision, int n, int c, const float* features, void* rows, void* stream);
+/* Stacked 3-NN, ref pointnet2_stack three_nn_wrapper (interpolate.cpp, interpolate_gpu.cu): unknown (N,3), known (M,3),
+ *      unknown_batch_cnt / known_batch_cnt (B) int32 on the device -> dist2 (N,3) f32 squared distances, idx (N,3) int32
+ *      GLOBAL known rows.  Row p belongs to the first frame k with p < N0+..+Nk (the search stops at B-1); ties keep the
+ *      smaller index; slots a frame with < 3 known points cannot fill are (+inf, the frame's known start).  One uniform
+ *      grid per frame (TSMDET_NN_ALGO=brute: none); no host synchronisation. */
+int tsmdet_stack_three_nn(int b, int n, int m, const float* unknown, const int* unknown_batch_cnt, const float* known,
+                          const int* known_batch_cnt, float* dist2, int* idx, void* stream);
+/* ref three_interpolate_wrapper (stack): features (M,C), idx / weight (N,3) -> out (N,C) (planes = 0) or (C,N)
+ *      (planes != 0), out = fmaf(w2,f2, fmaf(w0,f0, w1*f1)) per element; an index outside [0,M) reads 0. */
+int tsmdet_stack_three_interpolate(int n, int c, int m, const float* features, const int* idx, const float* weight,
+                                   float* out, int planes, void* stream);
+/* ref three_interpolate_grad_wrapper (stack): grad_out (N,C) -> grad_features (M,C) += g*w (atomic, zeroed by the
+ *      caller); indices outside [0,M) are skipped. */
+int tsmdet_stack_three_interpolate_grad(int n, int c, int m, const float* grad_out, const int* idx, const float* weight,
+                                        float* grad_features, void* stream);
 
 /* ---------------------------------------------------------------- IoU / NMS ---------
  * boxes (N,7) f32 [x,y,z,dx,dy,dz,heading] on the device.

@@ -584,6 +584,21 @@ int tsm_ball_query_grid(bool dilated, int b, int n, int m, float rin, float rout
     return TSM_OK;
 }
 
+int tsm_grid_build_ragged(int b, int n_total, float rout, const int* start, const float* xyz, cudaStream_t stream, int tag,
+                          const int** hdr_out, const int** cell_start_out, const float4** sorted_out) {
+    using namespace tsm;
+    GridScratch g;
+    const int rc = grid_scratch(tag, b, (size_t)n_total, stream, &g);
+    if (rc != TSM_OK) return rc;
+    TSM_CUDA_TRY(cudaFuncSetAttribute(bq_grid_build_ragged_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kBuildSmem));
+    bq_grid_build_ragged_kernel<<<b, 1024, kBuildSmem, stream>>>(rout, start, xyz, g.hdr, g.cell_start, g.tmp, g.sorted);
+    TSM_LAUNCH_CHECK();
+    *hdr_out = g.hdr;
+    *cell_start_out = g.cell_start;
+    *sorted_out = g.sorted;
+    return TSM_OK;
+}
+
 int tsm_stack_ball_query_grid(int b, int m, int n_total, float radius, int nsample, const float* new_xyz,
                               const int* mstart, const int* nstart, const float* xyz, int* idx, int* idx_cnt,
                               int global_rows, cudaStream_t stream, const int** grid_hdr) {
@@ -593,27 +608,25 @@ int tsm_stack_ball_query_grid(int b, int m, int n_total, float radius, int nsamp
     // frame then goes to the brute-force kernel)
     const float rout = fabsf(radius);
     if (!(rout > 0.f) || n_total <= 0) return TSM_OK;
-    GridScratch g;
-    const int rc = grid_scratch(9, b, (size_t)n_total, stream, &g);
+    const int *hdr = nullptr, *cell_start = nullptr;
+    const float4* sorted = nullptr;
+    const int rc = tsm_grid_build_ragged(b, n_total, rout, nstart, xyz, stream, 9, &hdr, &cell_start, &sorted);
     if (rc != TSM_OK) return rc;
-    TSM_CUDA_TRY(cudaFuncSetAttribute(bq_grid_build_ragged_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kBuildSmem));
-    bq_grid_build_ragged_kernel<<<b, 1024, kBuildSmem, stream>>>(rout, nstart, xyz, g.hdr, g.cell_start, g.tmp, g.sorted);
-    TSM_LAUNCH_CHECK();
     const float rout2 = radius * radius;  // f32 product, as ball_query_gpu.cu (stack):25
     if (nsample <= 32) {
         const unsigned blocks = (unsigned)((m + 15) / 16);
         if (nsample <= 16)
-            bq_grid_query16_ragged_kernel<1><<<blocks, 256, 0, stream>>>(b, m, rout2, nsample, new_xyz, mstart, nstart, g.hdr,
-                                                                         g.cell_start, g.sorted, idx_cnt, idx, global_rows);
+            bq_grid_query16_ragged_kernel<1><<<blocks, 256, 0, stream>>>(b, m, rout2, nsample, new_xyz, mstart, nstart, hdr,
+                                                                         cell_start, sorted, idx_cnt, idx, global_rows);
         else
-            bq_grid_query16_ragged_kernel<2><<<blocks, 256, 0, stream>>>(b, m, rout2, nsample, new_xyz, mstart, nstart, g.hdr,
-                                                                         g.cell_start, g.sorted, idx_cnt, idx, global_rows);
+            bq_grid_query16_ragged_kernel<2><<<blocks, 256, 0, stream>>>(b, m, rout2, nsample, new_xyz, mstart, nstart, hdr,
+                                                                         cell_start, sorted, idx_cnt, idx, global_rows);
     } else {
         bq_grid_merge_ragged_kernel<<<(unsigned)((m + 7) / 8), 256, 0, stream>>>(b, m, rout2, nsample, new_xyz, mstart, nstart,
-                                                                                 g.hdr, g.cell_start, g.sorted, idx_cnt, idx,
+                                                                                 hdr, cell_start, sorted, idx_cnt, idx,
                                                                                  global_rows);
     }
     TSM_LAUNCH_CHECK();
-    *grid_hdr = g.hdr;
+    *grid_hdr = hdr;
     return TSM_OK;
 }

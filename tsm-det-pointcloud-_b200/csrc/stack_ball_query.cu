@@ -75,6 +75,12 @@ __global__ void __launch_bounds__(256) stack_feature_rows_kernel(long long n, in
 
 }  // namespace tsm
 
+int tsm_stack_counts_scan(int b, const int* ncnt, const int* mcnt, int* nstart, int* mstart, cudaStream_t stream) {
+    tsm::stack_counts_scan_kernel<<<1, 64, 0, stream>>>(b, ncnt, mcnt, nstart, mstart);
+    TSM_LAUNCH_CHECK();
+    return TSM_OK;
+}
+
 extern "C" {
 
 int tsmdet_stack_ball_query(int b, int m, int n_total, float radius, int nsample, const float* new_xyz,
@@ -91,8 +97,8 @@ int tsmdet_stack_ball_query(int b, int m, int n_total, float radius, int nsample
     if (rc != TSM_OK) return rc;
     int* const nstart = static_cast<int*>(p);
     int* const mstart = nstart + b + 1;
-    stack_counts_scan_kernel<<<1, 64, 0, stream>>>(b, xyz_batch_cnt, new_xyz_batch_cnt, nstart, mstart);
-    TSM_LAUNCH_CHECK();
+    rc = tsm_stack_counts_scan(b, xyz_batch_cnt, new_xyz_batch_cnt, nstart, mstart, stream);
+    if (rc != TSM_OK) return rc;
     const int* ghdr = nullptr;
     const char* algo = tsm_knob(KNOB_BQ_ALGO);
     if (!(algo && !strcmp(algo, "brute"))) {

@@ -10,23 +10,24 @@
 // relative safety margin on that bound, far above the rounding of the cell coordinates) -- nothing outside the
 // cube can then enter the result, ties included.  Clouds whose grid is unusable are left to the brute-force
 // kernel (interpolate.cu), which skips the others.
+//
+// Stacked (ragged) frames, pointnet2_stack's three_nn: one grid per frame over its own known points
+// (tsm_grid_build_ragged, the build the stacked ball query uses) and three_nn_grid_ragged_kernel runs the same search
+// (three_nn_grid_core); it differs only in finding the unknown point's frame and in adding the frame's known start to
+// the indices.  Unusable frames go to stack_three_nn_kernel (stack_interpolate.cu).
 #include "grid.cuh"
 
 namespace tsm {
 
-__global__ void __launch_bounds__(256)
-    three_nn_grid_kernel(int n, int m, const float* __restrict__ unknown, const int* __restrict__ hdr_all,
-                         const int* __restrict__ cell_start_all, const float4* __restrict__ sorted_all,
-                         float* __restrict__ dist2, int* __restrict__ idx) {
-    const int b = blockIdx.y;
-    const GridHdr h = *reinterpret_cast<const GridHdr*>(hdr_all + (size_t)b * kHdrInts);
-    if (!h.ok) return;
-    const int i = blockIdx.x * 256 + threadIdx.x;
-    if (i >= n) return;
-    const int* __restrict__ cs = cell_start_all + (size_t)b * (kGridCells + 1);
-    const float4* __restrict__ sorted = sorted_all + (size_t)b * m;
-    const float* q = unknown + ((size_t)b * n + i) * 3;
-    const float ux = __ldg(q), uy = __ldg(q + 1), uz = __ldg(q + 2);
+// The three smallest (d2, k) pairs of the unknown point (ux, uy, uz) in one cloud's grid (cell starts cs, index-sorted
+// records `sorted` whose w holds the cloud-local index): (b1, i1) <= (b2, i2) <= (b3, i3), +inf / 0 past the cloud's
+// points.  The cloud's arrays come as base + offset, not as offset pointers: so three_nn_grid_kernel compiles to the same
+// SASS as before the core was factored out of it.
+__device__ __forceinline__ void three_nn_grid_core(const GridHdr& h, const int* cell_start_all, size_t cs_off,
+                                                   const float4* sorted_all, size_t s_off, float ux, float uy, float uz,
+                                                   float& b1, float& b2, float& b3, int& i1, int& i2, int& i3) {
+    const int* __restrict__ cs = cell_start_all + cs_off;
+    const float4* __restrict__ sorted = sorted_all + s_off;
     // cell coordinates (clamped) and the scaled position used for the face distances
     const float fx = __fmul_rn(__fsub_rn(ux, h.lo[0]), h.inv[0]);
     const float fy = __fmul_rn(__fsub_rn(uy, h.lo[1]), h.inv[1]);
@@ -35,8 +36,8 @@ __global__ void __launch_bounds__(256)
     const int cy = grid_q(uy, h.lo[1], h.inv[1], h.n[1]);
     const int cz = grid_q(uz, h.lo[2], h.inv[2], h.n[2]);
     const float inf = __int_as_float(0x7f800000);
-    float b1 = inf, b2 = inf, b3 = inf;  // (float)1e40 == +inf: what the reference's double 1e40 becomes in dist2
-    int i1 = 0, i2 = 0, i3 = 0;
+    b1 = inf; b2 = inf; b3 = inf;  // (float)1e40 == +inf: what the reference's double 1e40 becomes in dist2
+    i1 = 0; i2 = 0; i3 = 0;
 
     auto scan = [&](int s0, int s1) {
         for (int p = s0; p < s1; ++p) {
@@ -91,10 +92,54 @@ __global__ void __launch_bounds__(256)
             if (b3 < safe * safe) break;  // strictly closer than anything outside the cube: ties cannot come from there
         }
     }
+}
+
+__global__ void __launch_bounds__(256)
+    three_nn_grid_kernel(int n, int m, const float* __restrict__ unknown, const int* __restrict__ hdr_all,
+                         const int* __restrict__ cell_start_all, const float4* __restrict__ sorted_all,
+                         float* __restrict__ dist2, int* __restrict__ idx) {
+    const int b = blockIdx.y;
+    const GridHdr h = *reinterpret_cast<const GridHdr*>(hdr_all + (size_t)b * kHdrInts);
+    if (!h.ok) return;
+    const int i = blockIdx.x * 256 + threadIdx.x;
+    if (i >= n) return;
+    const float* q = unknown + ((size_t)b * n + i) * 3;
+    const float ux = __ldg(q), uy = __ldg(q + 1), uz = __ldg(q + 2);
+    float b1, b2, b3;
+    int i1, i2, i3;
+    three_nn_grid_core(h, cell_start_all, (size_t)b * (kGridCells + 1), sorted_all, (size_t)b * m, ux, uy, uz, b1, b2, b3,
+                       i1, i2, i3);
     float* od = dist2 + ((size_t)b * n + i) * 3;
     int* oi = idx + ((size_t)b * n + i) * 3;
     od[0] = b1; od[1] = b2; od[2] = b3;
     oi[0] = i1; oi[1] = i2; oi[2] = i3;
+}
+
+// Stacked (ragged) frames, pointnet2_stack's three_nn_kernel_stack contract: unknown row p belongs to frame
+// stack_frame_of(p) (ustart = the exclusive prefix sums of the unknown counts) and is answered from that frame's known
+// points; idx holds GLOBAL known rows (frame-local index + kstart[f]).  Frames whose grid is unusable are left to
+// stack_three_nn_kernel (stack_interpolate.cu).
+__global__ void __launch_bounds__(256)
+    three_nn_grid_ragged_kernel(int b, int n, const float* __restrict__ unknown, const int* __restrict__ ustart,
+                                const int* __restrict__ kstart, const int* __restrict__ hdr_all,
+                                const int* __restrict__ cell_start_all, const float4* __restrict__ sorted_all,
+                                float* __restrict__ dist2, int* __restrict__ idx) {
+    const int i = blockIdx.x * 256 + threadIdx.x;
+    if (i >= n) return;
+    const int f = stack_frame_of(i, b, ustart);
+    const GridHdr h = *reinterpret_cast<const GridHdr*>(hdr_all + (size_t)f * kHdrInts);
+    if (!h.ok) return;
+    const int start = __ldg(kstart + f);
+    const float* q = unknown + (size_t)i * 3;
+    const float ux = __ldg(q), uy = __ldg(q + 1), uz = __ldg(q + 2);
+    float b1, b2, b3;
+    int i1, i2, i3;
+    three_nn_grid_core(h, cell_start_all, (size_t)f * (kGridCells + 1), sorted_all, (size_t)start, ux, uy, uz, b1, b2, b3,
+                       i1, i2, i3);
+    float* od = dist2 + (size_t)i * 3;
+    int* oi = idx + (size_t)i * 3;
+    od[0] = b1; od[1] = b2; od[2] = b3;
+    oi[0] = i1 + start; oi[1] = i2 + start; oi[2] = i3 + start;
 }
 
 }  // namespace tsm
@@ -109,6 +154,21 @@ int tsm_three_nn_grid(int b, int n, int m, const float* unknown, const float* kn
     if (rc != TSM_OK) return rc;
     dim3 grid((unsigned)divup(n, 256), (unsigned)b);
     three_nn_grid_kernel<<<grid, 256, 0, stream>>>(n, m, unknown, hdr, cell_start, sorted, dist2, idx);
+    TSM_LAUNCH_CHECK();
+    *grid_hdr = hdr;
+    return TSM_OK;
+}
+
+// Stacked frames (grid.cuh); the grids use scratch tag 11, apart from the stacked ball query's 9.
+int tsm_stack_three_nn_grid(int b, int n, int m, const float* unknown, const int* ustart, const float* known,
+                            const int* kstart, float* dist2, int* idx, cudaStream_t stream, const int** grid_hdr) {
+    using namespace tsm;
+    const int *hdr = nullptr, *cell_start = nullptr;
+    const float4* sorted = nullptr;
+    int rc = tsm_grid_build_ragged(b, m, -1.f, kstart, known, stream, 11, &hdr, &cell_start, &sorted);
+    if (rc != TSM_OK) return rc;
+    three_nn_grid_ragged_kernel<<<(unsigned)divup(n, 256), 256, 0, stream>>>(b, n, unknown, ustart, kstart, hdr, cell_start,
+                                                                           sorted, dist2, idx);
     TSM_LAUNCH_CHECK();
     *grid_hdr = hdr;
     return TSM_OK;

@@ -1,6 +1,7 @@
-"""``StackSAModuleMSG`` of ``/root/reference/pcdet/ops/pointnet2/pointnet2_stack/pointnet2_modules.py`` (:11-94): the
-multi-scale set abstraction over stacked (ragged) frames that the VSA module of the detection head builds
-(``backbones_3d/pfe/voxel_set_abstraction.py``).
+"""``StackSAModuleMSG`` (:11-94) and ``StackPointnetFPModule`` of
+``/root/reference/pcdet/ops/pointnet2/pointnet2_stack/pointnet2_modules.py``: the multi-scale set abstraction over
+stacked (ragged) frames that the VSA module of the detection head builds (``backbones_3d/pfe/voxel_set_abstraction.py``),
+and the feature propagation that stacked backbones pair with it.
 
 Two execution modes give the same numbers within the tolerances of ``tests/parity.py``:
   ``fused=False`` (or train mode, or ``pool_method='avg_pool'``)  the reference's eager sequence: ``QueryAndGroup``
@@ -9,6 +10,9 @@ Two execution modes give the same numbers within the tolerances of ``tests/parit
                    SA kernel of the dense-batch module (gather + MLP + max-pool, BatchNorm folded): the stacked layout
                    seen as one cloud, xyz (1,N,3), new_xyz (1,M,3), idx (1,M,nsample), is exactly its input.
                    ``precision`` 'fp32' | 'bf16' | 'tf32' as for ``PointnetSAModuleFSMSG``.
+``StackPointnetFPModule`` likewise: eager (``fused=False`` or train mode) is the reference's sequence; in eval mode the
+stacked 3-NN feeds an interpolation kernel that writes the point-wise MLP's (1,C2,N) input planes, and the dense-batch
+FP module's fused MLP (``pointwise_mlp``) takes them with the skip features, never materialising the concatenation.
 """
 from __future__ import annotations
 
@@ -153,3 +157,89 @@ class StackSAModuleMSG(nn.Module):
                                   precision=precision, packed=img, feat_t=rows)
             c0 += w
         return out[0].t().contiguous()
+
+
+def _interp_weights(dist: torch.Tensor) -> torch.Tensor:
+    """inverse-distance weights of the three neighbours, normalised (ref StackPointnetFPModule.forward); 0/0 = NaN for an
+    unknown point whose frame has no known points"""
+    dist_recip = 1.0 / (dist + 1e-8)
+    norm = torch.sum(dist_recip, dim=-1, keepdim=True)
+    return dist_recip / norm
+
+
+def _dense_precision(precision: str, packed) -> str:
+    """The kernel an FP layer's MLP runs in: the point-wise tensor-core path takes exactly the shapes ``pack_mlp`` packs
+    (it has no first-generation fallback), so an MLP without a weight image, e.g. [768,512,512], runs in the fp32 FMA
+    kernel -- tighter, slower, never looser than asked for."""
+    return "fp32" if packed is None else precision
+
+
+class StackPointnetFPModule(nn.Module):
+    """ref StackPointnetFPModule: ``mlp`` = [C2 + C1, ...], [Conv2d 1x1 (no bias), BatchNorm2d, ReLU]* (state_dict keys
+    ``mlp.{3k}.weight``, ``mlp.{3k+1}.*``).  ``fused`` (eval mode only) and ``precision`` 'fp32' | 'bf16' | 'tf32' as for
+    the dense-batch ``PointnetFPModule``."""
+
+    def __init__(self, *, mlp: List[int], fused: bool = True, precision: str = "fp32"):
+        super().__init__()
+        self.mlp = _batch.build_shared_mlp(mlp, bn=True)
+        self.fused = fused
+        self.precision = precision
+        self._folded = None  # folded (W, b), built lazily in eval mode
+        self._packed = None
+
+    def train(self, mode: bool = True):
+        self._folded = None
+        return super().train(mode)
+
+    def _load_from_state_dict(self, *args, **kwargs):
+        self._folded = None  # the fused path must not keep running on the folds of the previous weights
+        return super()._load_from_state_dict(*args, **kwargs)
+
+    def _folded_layers(self):
+        if self._folded is None:
+            self._folded = _batch.fold_conv_bn(self.mlp)
+            self._packed = None
+        return self._folded
+
+    def _packed_layers(self, c2: int, c1: int):
+        folded = self._folded_layers()
+        if self._packed is None or self._packed[0] != (c2, c1, self.precision):
+            img = (_batch.pack_mlp(folded, dense=True, c_feat=c2, c1=c1, precision=self.precision)
+                   if self.precision in ("bf16", "tf32") else None)
+            self._packed = ((c2, c1, self.precision), img)
+        return self._packed[1]
+
+    def forward(self, unknown, unknown_batch_cnt, known, known_batch_cnt, unknown_feats=None, known_feats=None):
+        """unknown (N1+N2..., 3), unknown_batch_cnt (B), known (M1+M2..., 3), known_batch_cnt (B),
+        unknown_feats (N1+N2..., C1) | None, known_feats (M1+M2..., C2) -> (N1+N2..., mlp[-1])"""
+        if self.fused and not self.training:
+            return self._forward_fused(unknown, unknown_batch_cnt, known, known_batch_cnt, unknown_feats, known_feats)
+        dist, idx = pointnet2_utils.three_nn(unknown, unknown_batch_cnt, known, known_batch_cnt)
+        weight = _interp_weights(dist)
+        interpolated_feats = pointnet2_utils.three_interpolate(known_feats, idx, weight)
+        if unknown_feats is not None:
+            new_features = torch.cat([interpolated_feats, unknown_feats], dim=1)  # (N1 + N2 ..., C2 + C1)
+        else:
+            new_features = interpolated_feats
+        new_features = new_features.permute(1, 0)[None, :, :, None]  # (1, C, N1 + N2 ..., 1)
+        new_features = self.mlp(new_features)
+        return new_features.squeeze(dim=0).squeeze(dim=-1).permute(1, 0)  # (N1 + N2 ..., C)
+
+    @torch.no_grad()
+    def _forward_fused(self, unknown, unknown_batch_cnt, known, known_batch_cnt, unknown_feats, known_feats):
+        dist, idx = pointnet2_utils.three_nn(unknown, unknown_batch_cnt, known, known_batch_cnt)
+        weight = _interp_weights(dist)  # the eager path's weights, bit for bit
+        known_feats = known_feats.contiguous()
+        n, (m, c2) = unknown.shape[0], known_feats.shape
+        c1 = 0 if unknown_feats is None else unknown_feats.shape[1]
+        planes = torch.empty((1, c2, n), dtype=torch.float32, device=unknown.device)
+        call("tsmdet_stack_three_interpolate", n, c2, m, ptr(known_feats), ptr(idx), ptr(weight.contiguous()),
+             ptr(planes), 1, stream_ptr(unknown.device))
+        skip = None if unknown_feats is None else unknown_feats.t().contiguous().view(1, c1, n)
+        packed = self._packed_layers(c2, c1)
+        out = _batch.pointwise_mlp(planes, skip, self._folded, precision=_dense_precision(self.precision, packed),
+                                   packed=packed)
+        # a frame without known points has 0/0 weights: the eager path's rows are NaN there, whatever the MLP's ReLU
+        # makes of a NaN input
+        w0 = weight[:, :1]
+        return torch.where(torch.isnan(w0), w0, out[0].t()).contiguous()

@@ -64,3 +64,26 @@ def stack_farthest_point_sampling_wrapper(points, temp, xyz_batch_cnt, idx, num_
     call("tsmdet_stack_farthest_point_sampling", points.shape[0], xyz_batch_cnt.shape[0], ptr(points), ptr(temp),
          ptr(xyz_batch_cnt), ptr(idx), ptr(num_sampled_points), stream_ptr(points.device))
     return 1
+
+
+def three_nn_wrapper(unknown, unknown_batch_cnt, known, known_batch_cnt, dist2, idx):
+    """ref interpolate.cpp (stack): unknown (N,3), known (M,3) stacked, counts (B) int32 -> dist2 (N,3) squared
+    distances, idx (N,3) int32 GLOBAL known rows; slots a frame with < 3 known points cannot fill are (inf, its start)"""
+    _chk(unknown, unknown_batch_cnt, known, known_batch_cnt, dist2, idx)
+    call("tsmdet_stack_three_nn", unknown_batch_cnt.shape[0], unknown.shape[0], known.shape[0], ptr(unknown),
+         ptr(unknown_batch_cnt), ptr(known), ptr(known_batch_cnt), ptr(dist2), ptr(idx), stream_ptr(unknown.device))
+
+
+def three_interpolate_wrapper(features, idx, weight, out):
+    """features (M,C), idx / weight (N,3) -> out (N,C); an index outside [0, M) reads 0 (the reference reads out of
+    bounds there)"""
+    _chk(features, idx, weight, out)
+    call("tsmdet_stack_three_interpolate", idx.shape[0], features.shape[1], features.shape[0], ptr(features), ptr(idx),
+         ptr(weight), ptr(out), 0, stream_ptr(features.device))
+
+
+def three_interpolate_grad_wrapper(grad_out, idx, weight, grad_features):
+    """grad_out (N,C) -> grad_features (M,C) += g * w, zeroed by the caller"""
+    _chk(grad_out, idx, weight, grad_features)
+    call("tsmdet_stack_three_interpolate_grad", idx.shape[0], grad_out.shape[1], grad_features.shape[0], ptr(grad_out),
+         ptr(idx), ptr(weight), ptr(grad_features), stream_ptr(grad_out.device))

@@ -1,7 +1,7 @@
 """``BallQuery`` / ``QueryAndGroup`` / ``GroupingOperation`` / ``StackFarthestPointSampling`` /
-``FarthestPointSampling`` of ``/root/reference/pcdet/ops/pointnet2/pointnet2_stack/pointnet2_utils.py`` (:10-105,
-158-222) on the sm_100a kernels: same signatures, argument checks and returns (the 3-NN and vector-pool ops of that
-file are not part of this package)."""
+``FarthestPointSampling`` / ``ThreeNN`` / ``ThreeInterpolate`` of
+``/root/reference/pcdet/ops/pointnet2/pointnet2_stack/pointnet2_utils.py`` on the sm_100a kernels: same signatures,
+argument checks and returns (the vector-pool ops of that file are not part of this package)."""
 from __future__ import annotations
 
 import torch
@@ -156,3 +156,55 @@ class QueryAndGroup(nn.Module):
             assert self.use_xyz, "Cannot have not features and not use xyz as a feature!"
             new_features = grouped_xyz
         return new_features, idx
+
+
+class ThreeNN(Function):
+    """ref ThreeNN (stack)"""
+
+    @staticmethod
+    def forward(ctx, unknown, unknown_batch_cnt, known, known_batch_cnt):
+        """unknown (N1+N2..., 3), unknown_batch_cnt (B), known (M1+M2..., 3), known_batch_cnt (B)
+        -> (dist (N1+N2..., 3) l2 distances to the three nearest known points of the same frame,
+            idx (N1+N2..., 3) int32 GLOBAL known rows)"""
+        assert unknown.shape.__len__() == 2 and unknown.shape[1] == 3
+        assert known.shape.__len__() == 2 and known.shape[1] == 3
+        assert unknown_batch_cnt.__len__() == known_batch_cnt.__len__()
+
+        dist2 = unknown.new_zeros(unknown.shape)
+        idx = unknown_batch_cnt.new_zeros(unknown.shape).int()
+        pointnet2.three_nn_wrapper(unknown.contiguous(), unknown_batch_cnt.contiguous(), known.contiguous(),
+                                   known_batch_cnt.contiguous(), dist2, idx)
+        return torch.sqrt(dist2), idx
+
+    @staticmethod
+    def backward(ctx, a=None, b=None):
+        return None, None
+
+
+three_nn = ThreeNN.apply
+
+
+class ThreeInterpolate(Function):
+    """ref ThreeInterpolate (stack)"""
+
+    @staticmethod
+    def forward(ctx, features: torch.Tensor, idx: torch.Tensor, weight: torch.Tensor):
+        """features (M1+M2..., C), idx / weight (N1+N2..., 3) -> (N1+N2..., C)"""
+        assert idx.shape[0] == weight.shape[0] and idx.shape[1] == weight.shape[1] == 3
+
+        ctx.three_interpolate_for_backward = (idx, weight, features.shape[0])
+        output = features.new_zeros((idx.shape[0], features.shape[1]))
+        pointnet2.three_interpolate_wrapper(features.contiguous(), idx.contiguous(), weight.contiguous(), output)
+        return output
+
+    @staticmethod
+    def backward(ctx, grad_out: torch.Tensor):
+        """grad_out (N1+N2..., C) -> grad_features (M1+M2..., C)"""
+        idx, weight, M = ctx.three_interpolate_for_backward
+        grad_features = grad_out.new_zeros((M, grad_out.shape[1]))
+        pointnet2.three_interpolate_grad_wrapper(grad_out.contiguous(), idx.contiguous(), weight.contiguous(),
+                                                 grad_features)
+        return grad_features, None, None
+
+
+three_interpolate = ThreeInterpolate.apply
