@@ -260,6 +260,61 @@ int tsmdet_stack_three_interpolate(int n, int c, int m, const float* features, c
  *      caller); indices outside [0,M) are skipped. */
 int tsmdet_stack_three_interpolate_grad(int n, int c, int m, const float* grad_out, const int* idx, const float* weight,
                                         float* grad_features, void* stream);
+/* Vector pool (csrc/stack_vector_pool.cu; upstream OpenPCDet pointnet2_stack vector_pool_gpu.cu, restated there with
+ * what was recalled rather than read).  support_xyz (N,3) and new_xyz (M,3) stacked, xyz_batch_cnt / new_xyz_batch_cnt
+ * (B) i32 on the device, n_total = N; centre p belongs to the first frame k with p < M0+..+Mk.  A hit of centre p is a
+ * support point of its frame with local = support - centre (fp32 per axis) inside the ball (neighbor_type 1:
+ * fmaf(lz,lz, fmaf(lx,lx, ly*ly)) <= D*D) or the cube (otherwise: |l_a| <= D on every axis), D = max_neighbour_distance;
+ * hits are taken in ascending index.  One uniform grid per frame (TSMDET_BQ_ALGO=brute: none).
+ *
+ * query_stacked_local_neighbor_idxs_wrapper_stack: the first L = min(hits, 1000, nsample if > 0) hits of every centre as
+ *      GLOBAL rows; start_len (M,2) = (atomicAdd(cumsum, L), L); the list goes to stack_neighbor_idxs[offset..] except
+ *      entries at or beyond avg_length_of_neighbor_idxs * M.  *cumsum (device) is not zeroed here: it ends as its old
+ *      value plus the exact total of all L. */
+int tsmdet_stack_local_neighbor_idxs(int b, int m, int n_total, const float* support_xyz, const int* xyz_batch_cnt,
+                                     const float* new_xyz, const int* new_xyz_batch_cnt, int* stack_neighbor_idxs,
+                                     int* start_len, int* cumsum, int avg_length_of_neighbor_idxs,
+                                     float max_neighbour_distance, int nsample, int neighbor_type, void* stream);
+/* query_three_nn_by_stacked_local_idxs_wrapper_stack: for every (p, g), the three nearest (strict-< cascade in list
+ *      order, sqdist3) of centre p's list stack_neighbor_idxs[start_len[p,0] ..+ start_len[p,1]] (list_len entries exist;
+ *      the rest of a list is ignored) from new_xyz_grid_centers (M,G,3) -> new_xyz_grid_idxs (M,G,3) i32 GLOBAL rows and
+ *      new_xyz_grid_dist2 (M,G,3) f32; a slot the list cannot fill is (+inf, -1). */
+int tsmdet_stack_three_nn_local(int m, int num_total_grids, int n_total, long long list_len, const float* support_xyz,
+                                const float* new_xyz_grid_centers, const int* stack_neighbor_idxs, const int* start_len,
+                                int* new_xyz_grid_idxs, float* new_xyz_grid_dist2, void* stream);
+/* The two calls above in one, without the list: the same idx / dist2 as the list query (distance D, nsample,
+ *      neighbor_type) followed by the list 3-NN, bit for bit; no host synchronisation. */
+int tsmdet_stack_vector_three_nn(int b, int m, int n_total, int num_total_grids, const float* support_xyz,
+                                 const int* xyz_batch_cnt, const float* new_xyz, const int* new_xyz_batch_cnt,
+                                 const float* new_xyz_grid_centers, float max_neighbour_distance, int nsample,
+                                 int neighbor_type, int* new_xyz_grid_idxs, float* new_xyz_grid_dist2, void* stream);
+/* vector_pool_wrapper: G = num_grid_x*num_grid_y*num_grid_z sub-voxels per centre, cpg = c_out / G; a hit falls in
+ *      g = ix*ny*nz + iy*nz + iz (i_a = floorf((l_a + D) / (D*2 / num_grid_a)), fp32), clamped as one index to [0, G-1].
+ *      pooling_type 0 (average), per hit in index order: point_cnt_of_grid[p,g] += 1, new_features[p, g*cpg + i % cpg]
+ *      += support_features[k,i] (i ascending), new_local_xyz[p, 3g+a] += l_a if use_xyz, one triple (k, p, g) in
+ *      grouped_idxs; the hit counts toward nsample.  1 (random choice): only the first hit of each sub-voxel, assigned,
+ *      count 1; it stops when (nsample > 0 && taken >= nsample) || taken >= G.  The outputs are added to (and, random
+ *      choice, tested on) what the caller put there.  *num_cum_sum (device, zeroed here) = the exact number of triples;
+ *      those at or beyond num_max_sum_points are not written.  planes != NULL: no rows, counts or triples; instead
+ *      planes (1, G*(3+cpg), M) f32 = channel g*(3+cpg)+c of centre p: (c < 3 ? the local xyz sum c : the feature
+ *      sum c-3) / max((float)count, 1e-6f), the module's normalised eval input (use_xyz implied). */
+int tsmdet_stack_vector_pool(int b, int m, int n_total, int c_in, int c_out, const float* support_xyz,
+                             const int* xyz_batch_cnt, const float* support_features, const float* new_xyz,
+                             const int* new_xyz_batch_cnt, float* new_features, float* new_local_xyz,
+                             int* point_cnt_of_grid, int* grouped_idxs, int num_grid_x, int num_grid_y, int num_grid_z,
+                             float max_neighbour_distance, int use_xyz, long long num_max_sum_points, int nsample,
+                             int neighbor_type, int pooling_type, int* num_cum_sum, float* planes, void* stream);
+/* vector_pool_grad_wrapper: grad_support_features (N,c_in) (zeroed by the caller) += grad_new_features[p, g*cpg + i%cpg] *
+ *      (1 / max(point_cnt_of_grid[p,g], 1)) for every triple (k, p, g) of grouped_idxs (num_triples,3) (atomic). */
+int tsmdet_stack_vector_pool_grad(int m, int n, int c_out, int c_in, int num_total_grids, long long num_triples,
+                                  const float* grad_new_features, const int* point_cnt_of_grid, const int* grouped_idxs,
+                                  float* grad_support_features, void* stream);
+/* The local_interpolation eval input: planes (1, G*(C+9), M) f32, channel g*(C+9)+c of centre p for sub-voxel row
+ *      r = p*G+g: 0 if idx[r,0] == -1; else c < C: fmaf(w2,f2, fmaf(w0,f0, w1*f1)) (an index outside [0,N) reads 0),
+ *      c = C+3s+a: new_xyz_grid_centers[r,a] - support_xyz[idx[r,s], a], a -1 slot reading row N-1. */
+int tsmdet_stack_vector_interp_planes(int m, int num_total_grids, int n, int c, const float* support_features,
+                                      const float* support_xyz, const float* new_xyz_grid_centers, const int* idx,
+                                      const float* weight, float* planes, void* stream);
 
 /* ---------------------------------------------------------------- IoU / NMS ---------
  * boxes (N,7) f32 [x,y,z,dx,dy,dz,heading] on the device.

@@ -103,6 +103,19 @@ SIGNATURES = {
     "tsmdet_stack_three_nn": [c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p],
     "tsmdet_stack_three_interpolate": [c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p],
     "tsmdet_stack_three_interpolate_grad": [c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p],
+    "tsmdet_stack_local_neighbor_idxs": [c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                         c_void_p, c_int, c_float, c_int, c_int, c_void_p],
+    "tsmdet_stack_three_nn_local": [c_int, c_int, c_int, c_longlong, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                    c_void_p, c_void_p],
+    "tsmdet_stack_vector_three_nn": [c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_float,
+                                     c_int, c_int, c_void_p, c_void_p, c_void_p],
+    "tsmdet_stack_vector_pool": [c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                 c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_float, c_int, c_longlong,
+                                 c_int, c_int, c_int, c_void_p, c_void_p, c_void_p],
+    "tsmdet_stack_vector_pool_grad": [c_int, c_int, c_int, c_int, c_int, c_longlong, c_void_p, c_void_p, c_void_p,
+                                      c_void_p, c_void_p],
+    "tsmdet_stack_vector_interp_planes": [c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                          c_void_p, c_void_p],
     "tsmdet_boxes_overlap_bev": [c_int, c_void_p, c_int, c_void_p, c_void_p, c_void_p],
     "tsmdet_boxes_iou_bev": [c_int, c_void_p, c_int, c_void_p, c_void_p, c_void_p],
     "tsmdet_boxes_iou_bev_cpu": [c_int, c_void_p, c_int, c_void_p, c_void_p],
@@ -152,7 +165,8 @@ KERNELS_PER_CALL = {
     "tsmdet_fps_plan": 0, "tsmdet_fps_configure": 0, "tsmdet_enable_peer_access": 0, "tsmdet_read_status": 0,
     "tsmdet_reload_options": 0, "tsmdet_scratch_stats": 0, "tsmdet_scratch_trim": 0, "tsmdet_ball_query": 3, "tsmdet_ball_query_dilated": 3, "tsmdet_sa_mlp_maxpool": 3, "tsmdet_pointwise_mlp": 2, "tsmdet_sa_mlp_maxpool_packed": 2,
     "tsmdet_pointwise_mlp_packed": 1, "tsmdet_mlp_pack": 1, "tsmdet_sa_mlp_maxpool_packed_p": 2, "tsmdet_pointwise_mlp_packed_p": 1,
-    "tsmdet_mlp_pack_p": 1, "tsmdet_stack_ball_query": 4, "tsmdet_stack_three_nn": 4, "tsmdet_voxel_centroids": 2, "tsmdet_centroid_per_voxel": 2, "tsmdet_voxel2pinds": 2,
+    "tsmdet_mlp_pack_p": 1, "tsmdet_stack_ball_query": 4, "tsmdet_stack_three_nn": 4, "tsmdet_stack_local_neighbor_idxs": 3,
+    "tsmdet_stack_vector_three_nn": 3, "tsmdet_stack_vector_pool": 3, "tsmdet_voxel_centroids": 2, "tsmdet_centroid_per_voxel": 2, "tsmdet_voxel2pinds": 2,
 }
 launch_count = 0
 

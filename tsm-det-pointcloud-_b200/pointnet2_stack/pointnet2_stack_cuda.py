@@ -1,6 +1,6 @@
-"""Native surface of the reference's ``pointnet2_stack_cuda`` pybind module for the ops this package implements,
-re-hosted on the C ABI: same names / positional arguments / returns as
-``/root/reference/pcdet/ops/pointnet2/pointnet2_stack/src/pointnet2_api.cpp:13-20``."""
+"""Native surface of the reference's ``pointnet2_stack_cuda`` pybind module, every function it exports, re-hosted on
+the C ABI: same names / positional arguments / returns as
+``/root/reference/pcdet/ops/pointnet2/pointnet2_stack/src/pointnet2_api.cpp``."""
 from __future__ import annotations
 
 from .._lib import call, ptr, stream_ptr
@@ -87,3 +87,61 @@ def three_interpolate_grad_wrapper(grad_out, idx, weight, grad_features):
     _chk(grad_out, idx, weight, grad_features)
     call("tsmdet_stack_three_interpolate_grad", idx.shape[0], grad_out.shape[1], grad_features.shape[0], ptr(grad_out),
          ptr(idx), ptr(weight), ptr(grad_features), stream_ptr(grad_out.device))
+
+
+def query_stacked_local_neighbor_idxs_wrapper_stack(support_xyz, xyz_batch_cnt, new_xyz, new_xyz_batch_cnt,
+                                                    stack_neighbor_idxs, start_len, cumsum, avg_length_of_neighbor_idxs,
+                                                    max_neighbour_distance, nsample, neighbor_type):
+    """ref vector_pool.cpp: support_xyz (N,3), new_xyz (M,3) stacked, counts (B) int32 -> the first min(hits, 1000,
+    nsample if > 0) hits of every centre as GLOBAL rows, placed at start_len[p] = (atomicAdd(cumsum, L), L) in
+    stack_neighbor_idxs (nothing at or beyond avg_length_of_neighbor_idxs * M); cumsum (1) int32 ends as the total"""
+    _chk(support_xyz, xyz_batch_cnt, new_xyz, new_xyz_batch_cnt, stack_neighbor_idxs, start_len, cumsum)
+    call("tsmdet_stack_local_neighbor_idxs", xyz_batch_cnt.shape[0], new_xyz.shape[0], support_xyz.shape[0],
+         ptr(support_xyz), ptr(xyz_batch_cnt), ptr(new_xyz), ptr(new_xyz_batch_cnt), ptr(stack_neighbor_idxs),
+         ptr(start_len), ptr(cumsum), int(avg_length_of_neighbor_idxs), float(max_neighbour_distance), int(nsample),
+         int(neighbor_type), stream_ptr(support_xyz.device))
+    return 1
+
+
+def query_three_nn_by_stacked_local_idxs_wrapper_stack(support_xyz, new_xyz, new_xyz_grid_centers, new_xyz_grid_idxs,
+                                                       new_xyz_grid_dist2, stack_neighbor_idxs, start_len, M,
+                                                       num_total_grids):
+    """ref vector_pool.cpp: new_xyz_grid_centers (M,G,3) -> new_xyz_grid_idxs (M,G,3) int32 GLOBAL rows and
+    new_xyz_grid_dist2 (M,G,3), the three nearest of each centre's list; unfilled slots are (+inf, -1)"""
+    _chk(support_xyz, new_xyz, new_xyz_grid_centers, new_xyz_grid_idxs, new_xyz_grid_dist2, stack_neighbor_idxs,
+         start_len)
+    call("tsmdet_stack_three_nn_local", int(M), int(num_total_grids), support_xyz.shape[0], stack_neighbor_idxs.numel(),
+         ptr(support_xyz), ptr(new_xyz_grid_centers), ptr(stack_neighbor_idxs), ptr(start_len), ptr(new_xyz_grid_idxs),
+         ptr(new_xyz_grid_dist2), stream_ptr(support_xyz.device))
+    return 1
+
+
+def vector_pool_wrapper(support_xyz, xyz_batch_cnt, support_features, new_xyz, new_xyz_batch_cnt, new_features,
+                        new_local_xyz, point_cnt_of_grid, grouped_idxs, num_grid_x, num_grid_y, num_grid_z,
+                        max_neighbour_distance, use_xyz, num_max_sum_points, nsample, neighbor_type, pooling_type):
+    """ref vector_pool.cpp: sums (average, pooling_type 0) or first hits (random choice, 1) of every sub-voxel added to
+    new_features (M, G*cpg), new_local_xyz (M, 3G), point_cnt_of_grid (M,G) int32, triples (k, p, g) in grouped_idxs
+    (num_max_sum_points, 3) int32 -> the exact number of triples (a Python int: reads one int back from the device)"""
+    import torch
+
+    _chk(support_xyz, xyz_batch_cnt, support_features, new_xyz, new_xyz_batch_cnt, new_features, new_local_xyz,
+         point_cnt_of_grid, grouped_idxs)
+    total = torch.empty((1,), dtype=torch.int32, device=support_xyz.device)
+    call("tsmdet_stack_vector_pool", xyz_batch_cnt.shape[0], new_xyz.shape[0], support_xyz.shape[0],
+         support_features.shape[1], new_features.shape[1], ptr(support_xyz), ptr(xyz_batch_cnt), ptr(support_features),
+         ptr(new_xyz), ptr(new_xyz_batch_cnt), ptr(new_features), ptr(new_local_xyz), ptr(point_cnt_of_grid),
+         ptr(grouped_idxs), int(num_grid_x), int(num_grid_y), int(num_grid_z), float(max_neighbour_distance),
+         int(use_xyz), int(num_max_sum_points), int(nsample), int(neighbor_type), int(pooling_type), ptr(total), None,
+         stream_ptr(support_xyz.device))
+    return int(total.item())
+
+
+def vector_pool_grad_wrapper(grad_new_features, point_cnt_of_grid, grouped_idxs, grad_support_features):
+    """ref vector_pool.cpp: grad_support_features (N,C_in) (zeroed by the caller) += grad_new_features[p, g*cpg + i%cpg]
+    * (1 / max(point_cnt_of_grid[p,g], 1)) for every triple (k, p, g) of grouped_idxs (atomic)"""
+    _chk(grad_new_features, point_cnt_of_grid, grouped_idxs, grad_support_features)
+    call("tsmdet_stack_vector_pool_grad", grad_new_features.shape[0], grad_support_features.shape[0],
+         grad_new_features.shape[1], grad_support_features.shape[1], point_cnt_of_grid.shape[1], grouped_idxs.shape[0],
+         ptr(grad_new_features), ptr(point_cnt_of_grid), ptr(grouped_idxs), ptr(grad_support_features),
+         stream_ptr(grad_new_features.device))
+    return 1
