@@ -316,6 +316,30 @@ int tsmdet_stack_vector_interp_planes(int m, int num_total_grids, int n, int c, 
                                       const float* support_xyz, const float* new_xyz_grid_centers, const int* idx,
                                       const float* weight, float* planes, void* stream);
 
+/* ---------------------------------------------------------------- roiaware_pool3d ----
+ * Boxes / RoIs [cx, cy, cz, dx, dy, dz, heading] f32, (cx, cy, cz) the centre; the inside test is restated in
+ * csrc/roiaware_pool3d.cu (margin 1e-5 on the GPU, 1e-2 on the CPU; a NaN coordinate is never inside).
+ * ref: roiaware_pool3d/src/roiaware_pool3d.cpp (pybind names forward, backward, points_in_boxes_gpu,
+ *      points_in_boxes_cpu).  Sizes must be >= 0; every voxel grid dimension in [1, 256]; max_pts_each_voxel >= 1.
+ * points_in_boxes_gpu: boxes (B,T,7), pts (B,N,3), box_idx_of_points (B,N) i32 [in: the pre-fill, normally -1;
+ *      out: the first box holding the point, the pre-fill where none does]. */
+int tsmdet_points_in_boxes(int b, int t, int n, const float* boxes, const float* pts, int* box_idx_of_points,
+                           void* stream);
+/* points_in_boxes_cpu, HOST memory: boxes (M,7), pts (N,3) -> pts_indices (M,N) i32, 0 / 1 for every pair. */
+int tsmdet_points_in_boxes_cpu(int m, int n, const float* boxes, const float* pts, int* pts_indices);
+/* RoIAwarePool3d forward: rois (R,7), pts (P,3), pts_feature (P,C) -> pts_idx_of_voxels (R,X,Y,Z,L) i32 (slot 0 the
+ *      counter, at most L-1 points in ascending index; every counter written), argmax (R,X,Y,Z,C) i32 (max pool:
+ *      written everywhere, -1 for an empty voxel) and pooled_features (R,X,Y,Z,C) f32 (written for non-empty voxels
+ *      only: the caller zero-fills).  pool_method 0 max, 1 avg.  No allocation. */
+int tsmdet_roiaware_pool3d(int r, int p, int c, int out_x, int out_y, int out_z, int max_pts_each_voxel,
+                           const float* rois, const float* pts, const float* pts_feature, int* argmax,
+                           int* pts_idx_of_voxels, float* pooled_features, int pool_method, void* stream);
+/* RoIAwarePool3d backward: grad_in (P,C) (zeroed by the caller) += grad_out (R,X,Y,Z,C) at argmax (max) or
+ *      grad_out * (1 / max(count, 1)) at every listed point (avg); atomic. */
+int tsmdet_roiaware_pool3d_grad(int r, int p, int c, int out_x, int out_y, int out_z, int max_pts_each_voxel,
+                                const int* pts_idx_of_voxels, const int* argmax, const float* grad_out, float* grad_in,
+                                int pool_method, void* stream);
+
 /* ---------------------------------------------------------------- IoU / NMS ---------
  * boxes (N,7) f32 [x,y,z,dx,dy,dz,heading] on the device.
  * ref: iou3d_nms/src/iou3d_nms_api.cpp:12-13 boxes_overlap_bev_gpu / boxes_iou_bev_gpu

@@ -116,6 +116,12 @@ SIGNATURES = {
                                       c_void_p, c_void_p],
     "tsmdet_stack_vector_interp_planes": [c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                           c_void_p, c_void_p],
+    "tsmdet_points_in_boxes": [c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p],
+    "tsmdet_points_in_boxes_cpu": [c_int, c_int, c_void_p, c_void_p, c_void_p],
+    "tsmdet_roiaware_pool3d": [c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p,
+                               c_void_p, c_void_p, c_int, c_void_p],
+    "tsmdet_roiaware_pool3d_grad": [c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p,
+                                    c_void_p, c_int, c_void_p],
     "tsmdet_boxes_overlap_bev": [c_int, c_void_p, c_int, c_void_p, c_void_p, c_void_p],
     "tsmdet_boxes_iou_bev": [c_int, c_void_p, c_int, c_void_p, c_void_p, c_void_p],
     "tsmdet_boxes_iou_bev_cpu": [c_int, c_void_p, c_int, c_void_p, c_void_p],
@@ -167,6 +173,7 @@ KERNELS_PER_CALL = {
     "tsmdet_pointwise_mlp_packed": 1, "tsmdet_mlp_pack": 1, "tsmdet_sa_mlp_maxpool_packed_p": 2, "tsmdet_pointwise_mlp_packed_p": 1,
     "tsmdet_mlp_pack_p": 1, "tsmdet_stack_ball_query": 4, "tsmdet_stack_three_nn": 4, "tsmdet_stack_local_neighbor_idxs": 3,
     "tsmdet_stack_vector_three_nn": 3, "tsmdet_stack_vector_pool": 3, "tsmdet_voxel_centroids": 2, "tsmdet_centroid_per_voxel": 2, "tsmdet_voxel2pinds": 2,
+    "tsmdet_points_in_boxes_cpu": 0, "tsmdet_roiaware_pool3d": 2,
 }
 launch_count = 0
 
