@@ -190,7 +190,7 @@ enum TsmKnob {
     KNOB_BQ_ALGO, KNOB_FPS_CLUSTER, KNOB_FPS_THREADS, KNOB_FPS_ALGO, KNOB_FPSB_T,
     KNOB_FPSB_P, KNOB_FPSB_K, KNOB_GROUP_SLAB_KB, KNOB_GROUP_WAVES, KNOB_GROUP_DIRECT,
     KNOB_NN_ALGO, KNOB_NMS_CTAS_PER_SM, KNOB_NMS_ALGO, KNOB_MLP_ONE_GROUP, KNOB_MLP_OCC,
-    KNOB_MLP_V1, KNOB_FPSC_K, KNOB_VOXEL_ALGO, KNOB_MLP_NH,
+    KNOB_MLP_V1, KNOB_FPSC_K, KNOB_VOXEL_ALGO, KNOB_MLP_NH, KNOB_MLP_WIDTH,
     KNOB_COUNT
 };
 const char* tsm_knob(int id);

@@ -31,6 +31,7 @@
 // One CTA = GROUPS x 256 threads; a group = one independent 128-row tile pipeline (own operand buffer, TMEM
 // columns, mbarrier, named barrier) over the CTA's resident weights, persistent over tiles.
 #include <cstdio>
+#include <cstring>
 #include <type_traits>
 
 #include "sa_mlp.cuh"
@@ -73,7 +74,61 @@ struct Tc2Plan {
     int grp_cols, tmem_cols;   // TMEM columns of one tile group / of the CTA (power of two >= 32)
     int mb;                    // 128-channel blocks of the (transposed) last layer
     int whole_tiles;           // SA mode: M % (centres per tile) == 0 -> a tile's centres share the frame, consecutive p
+    int cls_off;               // SA mode, width-class tiles: the tile table + per-group centre ids in shared memory, else -1
+    int ncls;                  // width classes: log2(nsample) + 1
 };
+
+// ---- Width-class tiles (SA mode).  A centre is computed on the first w = 2^k rows of its nsample (w <= nsample) when
+// every idx slot j >= w repeats one of slots 0 .. w-1: then the dropped rows are byte copies of kept rows (same
+// neighbour, same centre, same mask), and
+//  * each output element of a tcgen05.mma depends only on its own A row and the weights (the bitwise tests against
+//    TSMDET_MLP_WIDTH=fixed confirm this on the hardware), so a copied row yields the same activations through
+//    every layer -- the mid-layer biases are per row, the last layer's bias and ReLU come after the pool;
+//  * the max over a set is unchanged by dropping duplicates.
+// So the width-class path is bit-identical to the fixed-width one.  sa_width_classify_kernel takes the smaller of two
+// widths it can prove from the row itself: next_pow2(cnt) when slots cnt.. are the cyclic padding the batch ball query
+// writes (row[j] == row[j mod cnt]: every value lies in slots 0 .. cnt-1), and next_pow2(t) when slots t.. all repeat
+// slot 0 (padding with the first hit, and hand-made rows).  A row that fits neither keeps nsample; an empty ball (cnt
+// <= 0: every row zeroed) has width 1.  It writes, per class k, the centre ids of that class into region k of a list
+// (order within a class is arbitrary; empty balls as ~id), and the class sizes; a class-k tile holds 128 >> k centres,
+// w rows each, the last tile of a class may be partial.  Tiles run class by class; the table of tile ranges is built by
+// every CTA from the class sizes, on the device, so the step needs no host synchronisation.
+constexpr int T2_MAX_CLS = 8;     // nsample <= 128
+constexpr int T2_CLS_LIST = 32;   // ints before the lists: the class sizes
+__global__ void __launch_bounds__(256) sa_width_classify_kernel(const int* __restrict__ idx, const int* __restrict__ cnt,
+                                                                const int centres, const int ns, int* __restrict__ cls) {
+    __shared__ int s_n[T2_MAX_CLS], s_base[T2_MAX_CLS];
+    if (threadIdx.x < T2_MAX_CLS) s_n[threadIdx.x] = 0;
+    __syncthreads();
+    const int i = blockIdx.x * 256 + threadIdx.x;
+    int k = -1, v = 0;
+    if (i < centres) {
+        const int* r = idx + (size_t)i * ns;
+        const int c = cnt != nullptr ? min(__ldg(cnt + i), ns) : ns;
+        const int i0 = __ldg(r);
+        int t = 1;         // 1 + the last slot that differs from slot 0
+        bool cyc = c > 0;  // slots c.. are row[j mod c]
+        for (int j = 1; j < ns; ++j) {
+            const int x = __ldg(r + j);
+            if (x != i0) t = j + 1;
+            if (j >= c && cyc && x != __ldg(r + j % c)) cyc = false;
+        }
+        if (cyc && c < t) t = c;
+        const bool empty = c <= 0;
+        if (empty) t = 1;
+        k = 32 - __clz(t - 1);  // ceil(log2(t))
+        v = empty ? ~i : i;
+    }
+    const unsigned peers = __match_any_sync(FULL, k);
+    const int lane = threadIdx.x & 31, leader = __ffs(peers) - 1;
+    int wb = 0;
+    if (k >= 0 && lane == leader) wb = atomicAdd(&s_n[k], __popc(peers));
+    wb = __shfl_sync(FULL, wb, leader) + __popc(peers & ((1u << lane) - 1u));
+    __syncthreads();
+    if (threadIdx.x < T2_MAX_CLS && s_n[threadIdx.x] > 0) s_base[threadIdx.x] = atomicAdd(cls + threadIdx.x, s_n[threadIdx.x]);
+    __syncthreads();
+    if (k >= 0) cls[T2_CLS_LIST + (size_t)k * centres + s_base[k] + wb] = v;
+}
 
 // Weights (cout,cin) fp32 + bias -> the kernel's shared-memory image: per layer bf16 [K/8 (+2)][Npad][8] (UMMA K-major
 // core matrices; non-last layers end with the two planes of the bias step: input row K = bf16(b), row K+1 = bf16(b -
@@ -259,11 +314,26 @@ __device__ __forceinline__ void epi_mid_rt(int hw, uint32_t taddr, unsigned char
 // max over W consecutive registers starting at v[O] (W = 8, 16 or 32), FMNMX3 tree
 template <int O, int W>
 __device__ __forceinline__ float max_run(const uint32_t (&v)[32]) {
-    float m = max3(__uint_as_float(v[O]), __uint_as_float(v[O + 1]), __uint_as_float(v[O + 2]));
+    if constexpr (W == 1) {
+        return __uint_as_float(v[O]);
+    } else if constexpr (W == 2) {
+        return fmaxf(__uint_as_float(v[O]), __uint_as_float(v[O + 1]));
+    } else {
+        float m = max3(__uint_as_float(v[O]), __uint_as_float(v[O + 1]), __uint_as_float(v[O + 2]));
 #pragma unroll
-    for (int j = 3; j + 1 < W; j += 2) m = max3(m, __uint_as_float(v[O + j]), __uint_as_float(v[O + j + 1]));
-    if ((W & 1) == 0) m = fmaxf(m, __uint_as_float(v[O + W - 1]));
-    return m;
+        for (int j = 3; j + 1 < W; j += 2) m = max3(m, __uint_as_float(v[O + j]), __uint_as_float(v[O + j + 1]));
+        if ((W & 1) == 0) m = fmaxf(m, __uint_as_float(v[O + W - 1]));
+        return m;
+    }
+}
+
+// emit(column of the centre's first row, its max) for every W-column centre of 32 loaded columns starting at c0
+template <int W, int J = 0, class F>
+__device__ __forceinline__ void emit_runs(const uint32_t (&v)[32], int c0, F&& emit) {
+    if constexpr (J < 32 / W) {
+        emit(c0 + J * W, max_run<J * W, W>(v));
+        emit_runs<W, J + 1>(v, c0, emit);
+    }
 }
 
 // GROUPS: tile pipelines per CTA; a pipeline is 128 * NH threads = NH (1 or 2) per tile row: thread (row, h) drains
@@ -287,7 +357,8 @@ __device__ __forceinline__ float max_run(const uint32_t (&v)[32]) {
 template <int GROUPS, int SC, bool DENSE, int PF, int NH, int MINB, int EB, int CL = 1>
 __global__ void __launch_bounds__(128 * NH * GROUPS, MINB)
     mlp_tc2_kernel(const __grid_constant__ SaMlpArgs a, const __grid_constant__ Tc2Plan pl,
-                   const unsigned char* __restrict__ featT, const unsigned char* __restrict__ packed, const int num_tiles) {
+                   const unsigned char* __restrict__ featT, const unsigned char* __restrict__ packed, const int fixed_tiles,
+                   const int* __restrict__ cls) {
     constexpr int EPC = 16 / EB;  // operand elements per 16-byte chunk
     static_assert(CL == 1 || (GROUPS == 1 && NH == 1 && !DENSE), "cluster pairs: one tile pipeline of 128 threads per CTA");
     const uint32_t crank = CL == 2 ? cluster_ctarank() : 0u;
@@ -309,18 +380,41 @@ __global__ void __launch_bounds__(128 * NH * GROUPS, MINB)
         else asm volatile("bar.sync %0, %1;" ::"r"(grp + 1), "n"(GT) : "memory");
     };
     const int S = a.s, M = a.m;
+    const int M_tot = (int)(a.total_rows >> (31 - __clz(S)));  // centres B*M: the stride of the class lists
     const int log2s = 31 - __clz(S);
     const int nl = pl.nl;
+
+    // width-class tiles: tt[k] = end of class k's tile range, tt[T2_MAX_CLS + k] = its number of centres
+    const bool classed = !DENSE && pl.cls_off >= 0;
+    int* const tt = reinterpret_cast<int*>(smem + (classed ? pl.cls_off : 0));
+    if (classed) {
+        if (threadIdx.x == 0) {
+            int end = 0;
+            for (int k = 0; k < pl.ncls; ++k) {
+                const int n = cls[k];
+                end += (n + (T2_ROWS >> k) - 1) >> (7 - k);
+                tt[k] = end;
+                tt[T2_MAX_CLS + k] = n;
+            }
+        }
+        __syncthreads();
+    }
+    const int num_tiles = classed ? tt[pl.ncls - 1] : fixed_tiles;
+    // A CTA whose tile groups all start past the last tile (width classes: the grid is sized for fixed-width tiles)
+    // neither copies the weights nor allocates TMEM.  (Tile t runs on CTA t % G, see tile0 below.)
+    const bool busy = (int)(blockIdx.x / CL) < num_tiles;
 
     // ---- one-time setup: weights + bias rows + ones operand arrive with ONE bulk copy (TMA engine); barriers; TMEM
     if (threadIdx.x == 0) {
         for (int g = 0; g < GROUPS; ++g) mbar_init(smem_u32(&mma_bars[g]), 1);
         mbar_init(smem_u32(&w_bar), 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        mbar_arrive_expect_tx(smem_u32(&w_bar), (uint32_t)pl.packed_bytes);
-        bulk_g2s(smem_u32(smem), packed + (size_t)crank * pl.packed_bytes, (uint32_t)pl.packed_bytes, smem_u32(&w_bar));
+        if (busy) {
+            mbar_arrive_expect_tx(smem_u32(&w_bar), (uint32_t)pl.packed_bytes);
+            bulk_g2s(smem_u32(smem), packed + (size_t)crank * pl.packed_bytes, (uint32_t)pl.packed_bytes, smem_u32(&w_bar));
+        }
     }
-    if (threadIdx.x < 32) {
+    if (busy && threadIdx.x < 32) {
         asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_s)),
                      "r"((uint32_t)pl.tmem_cols)
                      : "memory");
@@ -330,6 +424,13 @@ __global__ void __launch_bounds__(128 * NH * GROUPS, MINB)
     __syncthreads();
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     if constexpr (CL == 2) cluster_sync_all();  // the peer CTA is resident before anything is stored into it
+    // classed: tile -> its class k and the list position of its first centre
+    auto tile_class = [&](int tile, int& first) {
+        int k = 0;
+        while (k + 1 < pl.ncls && tile >= tt[k]) ++k;
+        first = (tile - (k > 0 ? tt[k - 1] : 0)) << (7 - k);
+        return k;
+    };
     bool weights_in = false;  // the weight image is awaited right before the first MMA: the first gather overlaps its copy
     auto wait_weights = [&]() {
         if (!weights_in) {
@@ -363,17 +464,34 @@ __global__ void __launch_bounds__(128 * NH * GROUPS, MINB)
     uint32_t phase = 0;
     const int cout_last = a.ch[nl];
     const int nchunk0 = pl.K[0] / EPC;
-    const int tile0 = (blockIdx.x / CL) * GROUPS + grp, tile_step = (gridDim.x / CL) * GROUPS;  // both CTAs of a pair: the same tiles
+    // tile t -> CTA t % G, group (t / G) % GROUPS (G = CTAs, or pairs): fewer tiles than groups (width classes) still
+    // land on as many SMs as there are tiles; both CTAs of a pair walk the same tiles
+    const int tile0 = grp * (int)(gridDim.x / CL) + (int)(blockIdx.x / CL), tile_step = (gridDim.x / CL) * GROUPS;
 
     // SA mode: the neighbour index and the hit count of this thread's row are LOADED one tile ahead and only looked at
     // when the next gather is issued; the coordinates are loaded when the gather is issued and only looked at when it
     // is finished -- no load is consumed where it is issued.
-    int id_raw = 0, cnt_raw = 1;
+    // Classed tiles: row r of a class-k tile is slot r % 2^k of centre list[first + r / 2^k] (cg_raw, -1 past the
+    // class's end); its neighbour index is loaded behind the list entry in the same prefetch.
+    int id_raw = 0, cnt_raw = 1, cg_raw = -1;
     auto prefetch_row = [&](int tile) {
         if constexpr (!DENSE) {
             id_raw = 0;
             cnt_raw = 0;  // rows past the end are masked
-            if (tile < num_tiles) {
+            cg_raw = -1;
+            if (classed) {
+                if (tile < num_tiles) {
+                    int first;
+                    const int k = tile_class(tile, first);
+                    const int pos = first + (row >> k);
+                    if (pos < tt[T2_MAX_CLS + k]) {
+                        const int v = __ldg(cls + T2_CLS_LIST + (size_t)k * M_tot + pos);
+                        cg_raw = v >= 0 ? v : ~v;
+                        cnt_raw = v >= 0 ? 1 : 0;
+                        id_raw = __ldg(a.idx + (size_t)cg_raw * S + (row & ((1 << k) - 1)));
+                    }
+                }
+            } else if (tile < num_tiles) {
                 const long long g = (long long)tile * T2_ROWS + row;
                 if (g < a.total_rows) {
                     id_raw = __ldg(a.idx + g);
@@ -405,7 +523,7 @@ __global__ void __launch_bounds__(128 * NH * GROUPS, MINB)
             const int id = id_raw;
             const bool live = cnt_raw > 0;
             pend_live = live;
-            const long long cpi = g < a.total_rows ? (g >> log2s) : 0;  // S is a power of two; B*M < 2^31 (launcher)
+            const long long cpi = classed ? (cg_raw >= 0 ? cg_raw : 0) : (g < a.total_rows ? (g >> log2s) : 0);  // S is a power of two; B*M < 2^31 (launcher)
             const int b = (int)((unsigned)cpi / (unsigned)M);
             const size_t prow = (size_t)b * a.n + id;
             if (own_xyz && live) {
@@ -782,30 +900,88 @@ __global__ void __launch_bounds__(128 * NH * GROUPS, MINB)
                             }
                         }
                     }
-                    if (NH == 2 && SC == 32 && S == 128) {  // uniform; the next write of xbuf lies behind the next tile's barriers
-                        float* const xbuf = reinterpret_cast<float*>(smem + pl.x_off) + grp * (2 * T2_ROWS);
-                        if (h == 1) {
-                            xbuf[row] = part0;
-                            xbuf[T2_ROWS + row] = part1;
-                        }
-                        group_sync();
-                        if (h == 0) {
-                            for (int mb = 0; mb < pl.mb; ++mb) {
-                                const int ch = mb * T2_ROWS + row;  // (NH == 2 excludes cluster pairs)
-                                const bool ch_ok = ch < cout_last;
-                                const float m = fmaxf(mb == 0 ? part0 : part1, xbuf[mb * T2_ROWS + row]);
-                                const float y = ch_ok ? fmaxf(__fadd_rn(m, bs[ch]), 0.f) : 0.f;
-                                if (cbase < ctot) {  // one centre per tile
-                                    if (a.out != nullptr && ch_ok) a.out[((size_t)b0 * a.out_ctot + a.out_c0 + ch) * M + p0] = y;
-                                    if (a.out_t != nullptr && ch < cpo)
-                                        reinterpret_cast<RowT*>(a.out_t)[(size_t)cbase * cpo + ch] = to_row(y);
+                };
+                int xk = log2s;  // log2 of this tile's rows per centre
+                if (classed) {
+                    // one 32-column load at a time; centre j of a class-k tile is list entry first + j, its rows are
+                    // columns j << k ..
+                    int first;
+                    xk = tile_class(tile, first);
+                    const int* const lst = cls + T2_CLS_LIST + (size_t)xk * M_tot + first;
+                    const int nlst = tt[T2_MAX_CLS + xk] - first;
+                    for (int mb = 0; mb < pl.mb; ++mb) {
+                        const int ch = (mb + (int)crank) * T2_ROWS + row;
+                        const float bias = bs[mb * T2_ROWS + row];
+                        const bool ch_ok = ch < cout_last;
+                        const bool o_ok = a.out != nullptr && ch_ok;
+                        const bool t_ok = a.out_t != nullptr && ch < cpo;
+                        auto emit = [&](int c, float m) {  // c: tile column of the centre's first row
+                            if ((c >> xk) >= nlst) return;  // past the end of the class
+                            const int v = __ldg(lst + (c >> xk));
+                            const int cg = v >= 0 ? v : ~v;
+                            const float y = ch_ok ? fmaxf(__fadd_rn(m, bias), 0.f) : 0.f;
+                            if (o_ok) {
+                                const unsigned b2 = (unsigned)cg / (unsigned)M, p2 = (unsigned)cg - b2 * (unsigned)M;
+                                a.out[((size_t)b2 * a.out_ctot + a.out_c0 + ch) * M + p2] = y;
+                            }
+                            if (t_ok) reinterpret_cast<RowT*>(a.out_t)[(size_t)cg * cpo + ch] = to_row(y);
+                        };
+                        if ((mb + (int)crank) * T2_ROWS + (row & ~31) >= (cpo > cout_last ? cpo : cout_last)) continue;  // warp-uniform: padding channels
+                        float run = 0.f;
+#pragma unroll 1
+                        for (int cb = 0; cb < PW; cb += 32) {
+                            const int c0 = PW * h + cb;
+                            uint32_t v[32];
+                            tmem_ld32_nowait(t_part + (uint32_t)(mb * T2_ROWS + cb), v);
+                            tmem_wait_ld();
+                            switch (xk) {
+                                case 0: emit_runs<1>(v, c0, emit); break;
+                                case 1: emit_runs<2>(v, c0, emit); break;
+                                case 2: emit_runs<4>(v, c0, emit); break;
+                                case 3: emit_runs<8>(v, c0, emit); break;
+                                case 4: emit_runs<16>(v, c0, emit); break;
+                                default: {  // 32, 64 or 128 rows per centre: the 32 columns lie inside one centre
+                                    const int w = 1 << xk;
+                                    const float m = max_run<0, 32>(v);
+                                    run = (cb == 0 || (c0 & (w - 1)) == 0) ? m : fmaxf(run, m);  // (a half: from its first column)
+                                    if (((c0 + 32) & (w - 1)) == 0 && w <= PW) emit(c0 + 32 - w, run);
                                 }
                             }
                         }
+                        if (mb == 0) part0 = run;  // 128 rows per centre, NH == 2: this half's maximum (below)
+                        else part1 = run;
                     }
-                };
-                if (full) pool(std::true_type{});
-                else pool(std::false_type{});
+                } else if (full) {
+                    pool(std::true_type{});
+                } else {
+                    pool(std::false_type{});
+                }
+                if (NH == 2 && SC == 32 && xk == 7) {  // uniform; the next write of xbuf lies behind the next tile's barriers
+                    float* const xbuf = reinterpret_cast<float*>(smem + pl.x_off) + grp * (2 * T2_ROWS);
+                    if (h == 1) {
+                        xbuf[row] = part0;
+                        xbuf[T2_ROWS + row] = part1;
+                    }
+                    group_sync();
+                    int cg = cbase < ctot ? (int)cbase : -1;  // one centre per tile
+                    if (classed) {
+                        int first;
+                        tile_class(tile, first);
+                        const int v = __ldg(cls + T2_CLS_LIST + (size_t)7 * M_tot + first);
+                        cg = v >= 0 ? v : ~v;
+                    }
+                    if (h == 0 && cg >= 0) {
+                        const unsigned b2 = (unsigned)cg / (unsigned)M, p2 = (unsigned)cg - b2 * (unsigned)M;
+                        for (int mb = 0; mb < pl.mb; ++mb) {
+                            const int ch = mb * T2_ROWS + row;  // (NH == 2 excludes cluster pairs)
+                            const bool ch_ok = ch < cout_last;
+                            const float m = fmaxf(mb == 0 ? part0 : part1, xbuf[mb * T2_ROWS + row]);
+                            const float y = ch_ok ? fmaxf(__fadd_rn(m, bs[ch]), 0.f) : 0.f;
+                            if (a.out != nullptr && ch_ok) a.out[((size_t)b2 * a.out_ctot + a.out_c0 + ch) * M + p2] = y;
+                            if (a.out_t != nullptr && ch < cpo) reinterpret_cast<RowT*>(a.out_t)[(size_t)cg * cpo + ch] = to_row(y);
+                        }
+                    }
+                }
                 // no barrier here: the next tile's MMA is issued after the barrier that follows store_row()
             } else {
                 // dense: thread = (output channel, half): 64 columns = 64 consecutive rows (points) of the tile
@@ -882,7 +1058,7 @@ __global__ void __launch_bounds__(128 * NH * GROUPS, MINB)
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
     if constexpr (CL == 2) cluster_sync_all();  // no CTA leaves while its peer may still store into it
-    if (threadIdx.x < 32) {
+    if (busy && threadIdx.x < 32) {
         asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base_s), "r"((uint32_t)pl.tmem_cols)
                      : "memory");
     }
@@ -963,6 +1139,8 @@ static int tc2_plan_cl(const tsm::SaMlpArgs& a, long long centres, int dense, in
     pl.tmem_cols = pl.grp_cols * groups;
     pl.x_off = xch ? off + groups * pl.a_bytes : -1;
     pl.smem_bytes = smem_for(groups);
+    pl.cls_off = -1;  // set by the launcher when width-class tiles fit behind the plan (tc2_classed)
+    pl.ncls = 0;
     *out = pl;
     *groups_out = groups;
     return TSM_OK;
@@ -974,6 +1152,21 @@ static int tc2_plan(const tsm::SaMlpArgs& a, long long centres, int dense, int e
     int rc = tc2_plan_cl(a, centres, dense, eb, 1, out, groups_out);
     if (rc == TSM_ERR_INVALID && eb == 4 && !dense) rc = tc2_plan_cl(a, centres, dense, eb, 2, out, groups_out);
     return rc;
+}
+
+// Width-class tiles for an SA scale: the 64-byte tile table goes behind the plan's shared memory (the plan itself --
+// weight image, groups, cluster pair -- stays as for fixed-width tiles, which the call keeps where the table does
+// not fit or would cost a resident CTA).  TSMDET_MLP_WIDTH=fixed: always fixed-width tiles; =classes: a call the width
+// classes do not take fails (TSM_ERR_INVALID) instead -- tests use it to know which path they compared.
+static bool tc2_classed(tsm::Tc2Plan& pl, int nsample) {
+    using namespace tsm;
+    const int bytes = 2 * T2_MAX_CLS * 4;
+    if (pl.smem_bytes + bytes > 227 * 1024 - 64) return false;
+    if ((227 * 1024) / (pl.smem_bytes + bytes + 2048) < (227 * 1024) / (pl.smem_bytes + 2048)) return false;
+    pl.cls_off = pl.smem_bytes;
+    pl.smem_bytes += bytes;
+    pl.ncls = 32 - __builtin_clz((unsigned)nsample);  // nsample = 2^(ncls - 1)
+    return true;
 }
 
 // The kernel's weight image (bf16 UMMA core matrices incl. the bias steps, the last fp32 bias, the ones operand) for an
@@ -1033,9 +1226,25 @@ int tsm_mlp_tc2(const tsm::SaMlpArgs& a, int b, int dense, int eb, cudaStream_t 
         }
         TSM_LAUNCH_CHECK();
     }
+    // fixed-width tiles; the grid is sized for them.  (Width classes make up to ncls - 1 more tiles when all classes end
+    // in partial tiles -- the persistent loop takes any count.)
     const long long tiles = (a.total_rows + T2_ROWS - 1) / T2_ROWS;
     if (tiles > 0x7fffffffLL) return TSM_ERR_INVALID;
-    using Kern = void (*)(const SaMlpArgs, const Tc2Plan, const unsigned char*, const unsigned char*, const int);
+    int* cls = nullptr;
+    const char* wk = dense ? nullptr : tsm_knob(KNOB_MLP_WIDTH);
+    const bool want_classes = !dense && !(wk && strcmp(wk, "fixed") == 0);
+    if (want_classes && !tc2_classed(pl, S) && wk && strcmp(wk, "classes") == 0) return TSM_ERR_INVALID;
+    if (pl.cls_off >= 0) {
+        const long long centres = (long long)b * a.m;
+        void* p = nullptr;
+        int rc = tsm_scratch_get(15, (T2_CLS_LIST + (size_t)pl.ncls * centres) * sizeof(int), stream, &p);
+        if (rc != TSM_OK) return rc;
+        cls = static_cast<int*>(p);
+        TSM_CUDA_TRY(cudaMemsetAsync(cls, 0, T2_CLS_LIST * sizeof(int), stream));
+        sa_width_classify_kernel<<<(unsigned)divup((int)centres, 256), 256, 0, stream>>>(a.idx, a.idx_cnt, (int)centres, S, cls);
+        TSM_LAUNCH_CHECK();
+    }
+    using Kern = void (*)(const SaMlpArgs, const Tc2Plan, const unsigned char*, const unsigned char*, const int, const int*);
     Kern kern = nullptr;
     // threads per tile row (see the kernel's comment), TSMDET_MLP_NH=1|2 overrides (bf16 SA scales only)
     int nh = dense ? 2 : 1;  // measured (B200, config 2 / config 4): SA L1/L2/L3 48/36/50 us vs 74/48/60, FP MLP 285 vs 233 us
@@ -1124,9 +1333,9 @@ int tsm_mlp_tc2(const tsm::SaMlpArgs& a, int b, int dense, int eb, cudaStream_t 
         cfg.attrs = attr;
         cfg.numAttrs = 1;
         const int ntiles = (int)tiles;
-        TSM_CUDA_TRY(cudaLaunchKernelEx(&cfg, kern, args, pl, featT, packed, ntiles));
+        TSM_CUDA_TRY(cudaLaunchKernelEx(&cfg, kern, args, pl, featT, packed, ntiles, (const int*)cls));
     } else {
-        kern<<<(unsigned)grid, gthreads * groups, pl.smem_bytes, stream>>>(args, pl, featT, packed, (int)tiles);
+        kern<<<(unsigned)grid, gthreads * groups, pl.smem_bytes, stream>>>(args, pl, featT, packed, (int)tiles, cls);
     }
     TSM_LAUNCH_CHECK();
     return TSM_OK;

@@ -17,7 +17,7 @@ static const char* const kKnobNames[KNOB_COUNT] = {
     "TSMDET_BQ_ALGO",       "TSMDET_FPS_CLUSTER",  "TSMDET_FPS_THREADS",     "TSMDET_FPS_ALGO",   "TSMDET_FPSB_T",
     "TSMDET_FPSB_P",        "TSMDET_FPSB_K",       "TSMDET_GROUP_SLAB_KB",   "TSMDET_GROUP_WAVES", "TSMDET_GROUP_DIRECT",
     "TSMDET_NN_ALGO",       "TSMDET_NMS_CTAS_PER_SM", "TSMDET_NMS_ALGO",     "TSMDET_MLP_ONE_GROUP", "TSMDET_MLP_OCC",
-    "TSMDET_MLP_V1",        "TSMDET_FPSC_K",       "TSMDET_VOXEL_ALGO",      "TSMDET_MLP_NH",
+    "TSMDET_MLP_V1",        "TSMDET_FPSC_K",       "TSMDET_VOXEL_ALGO",      "TSMDET_MLP_NH",     "TSMDET_MLP_WIDTH",
 };
 static std::string g_knob_val[KNOB_COUNT];
 static bool g_knob_set[KNOB_COUNT];
