@@ -615,7 +615,10 @@ __global__ void __launch_bounds__(T, 1)
                 // is the update's own expression on the candidate, evaluated by every lane alike (no vote).
                 const float cx = sx[wpos & 0x7fffffffu], cy = sy[wpos & 0x7fffffffu], cz = sz[wpos & 0x7fffffffu];
                 const float cval = __uint_as_float(wu & 0x7fffffffu);
-                bool redo = (wu & 0x80000000u) == 0u;  // no valid record yet (first round, ineligible warp)
+                // no valid record yet (first round, ineligible warp), or a hit record that says a point with different
+                // coordinates shares its maximum: that point may just have been lowered, and a stale bit would record a
+                // tie the one-pick algorithm never sees (tie_iter too early, chained shortcut lost)
+                bool redo = (wu & 0x80000000u) == 0u || (wpos >> 31) != 0u;
 #ifdef FPSB_PROF
                 const long long pwc = clock_after(__float_as_uint(cx) ^ __float_as_uint(cy) ^ __float_as_uint(cz));
                 pw_c += pwc - pw0;
@@ -775,8 +778,10 @@ __global__ void __launch_bounds__(T, 1)
                     run2 = max(run2, 4 * q + 3 < lane ? v.w : 0u);
                 }
                 // keys of positive finite values lie in (0x80000000, 0xff800000); anything else ends the round
+                // (and a later record whose maximum a point with different coordinates shares: an earlier pick of the
+                // round may lower that point, after which the one-pick algorithm records no tie)
                 const bool ok = lane == 0 || (valid && !near_tie && j + lane < m && qkey > run2 && qkey > 0x80000000u &&
-                                              qkey < 0xff800000u && !moved);
+                                              qkey < 0xff800000u && !moved && (qpos >> 31) == 0u);
                 PROF_TD(tq3, (ok ? 1u : 0u));
                 const unsigned okm = __ballot_sync(FULL, ok);
                 const int cnt = __ffs(~okm) - 1;  // the leading run of accepted positions
